@@ -56,6 +56,30 @@ def qber_grid():
     return [0.03 + 0.01 * j for j in range(9)]  # end-exclusive grid of src/simulation.cpp:55-61 for 0.03..0.12 step 0.01
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, iterations, flags):
+    """--dump-outputs: what the last timed step returned, for comparing two builds output for output. iterations.npy and
+    result_flags.npy (bit 0 syndromes match, bit 1 keys match) are float32 [QBER points x frames]; point_stats.npy is float64
+    [points x sweep.PointStats]; frame_index.npy lists the frames kept. Above 64 MB the frames are a fixed, seeded sample."""
+    from qkd_ldpc_b200 import sweep
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    points, frames = iterations.shape
+    stats = np.zeros((points, MAX_IT + 5), np.float64)
+    for pt in range(points):
+        ps = sweep.PointStats(MAX_IT)
+        ps.add(iterations[pt], flags[pt])
+        stats[pt] = ps.vec
+    keep = (DUMP_LIMIT_BYTES - stats.nbytes - 4096) // (2 * 4 * points + 8)
+    idx = np.arange(frames) if frames <= keep else np.sort(np.random.default_rng(0).choice(frames, keep, replace=False))
+    np.save(out / "iterations.npy", iterations[:, idx].astype(np.float32))
+    np.save(out / "result_flags.npy", flags[:, idx].astype(np.float32))
+    np.save(out / "frame_index.npy", idx.astype(np.float64))
+    np.save(out / "point_stats.npy", stats)
+
+
 def measured_peaks():
     p = ROOT / "MEASURED_PEAKS.json"
     if p.exists():
@@ -175,6 +199,8 @@ def run_reference_arm(args, guard):
         "per_qber": [{"qber": q, "fer": f} for q, f in zip(grid, fer)],
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.stack([o[:, 0] for o in outs]), np.stack([o[:, 1] | (o[:, 2] << np.uint64(1)) for o in outs]))
     guard.emit(line)
     return 0
 
@@ -230,7 +256,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-frame outputs of the last timed step to DIR/*.npy (rank 0; the inputs are fixed by the seeds)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "b200":
         args.warmup = max(args.warmup, 3)
 
@@ -624,6 +654,8 @@ def main():
             "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu, "clocks": clocks,
             "parity": parity, "per_qber": per_qber, "fer_parity_vs_cpu_sample": fer_parity, "strong": strong, "variants": variants,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *outcomes[prec])
         guard.emit(line)
     if world > 1:
         dist.destroy_process_group()

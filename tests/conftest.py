@@ -24,15 +24,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def reference():
-    """The unmodified reference compiled in place; only available where oracle/_ref was built."""
-    from oracle.bindings import REF_SO, REFERENCE_ROOT, Reference
-    if not REF_SO.exists() and not (REFERENCE_ROOT / "src").exists():
-        pytest.skip("oracle/_ref is not built and /root/reference is absent")
-    return Reference()
-
-
-@pytest.fixture(scope="session")
 def matrices():
     from qkd_ldpc_b200 import codes
     return {p.stem: codes.load_npz(p) for p in sorted(codes.CODES.glob("*.npz"))}
