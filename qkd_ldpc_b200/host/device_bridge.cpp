@@ -134,17 +134,4 @@ namespace qkd_b200
             p.flags |= QLB_FLAG_F64_FUSED_RATIO;
         return p;
     }
-
-    void pack_bits(const int *bits, size_t n, uint32_t *words_out)
-    {
-        const size_t words = (n + 31) / 32;
-        for (size_t w = 0; w < words; ++w)
-        {
-            uint32_t v = 0;
-            const size_t lim = std::min<size_t>(32, n - w * 32);
-            for (size_t b = 0; b < lim; ++b)
-                v |= static_cast<uint32_t>(bits[w * 32 + b] & 1) << b;
-            words_out[w] = v;
-        }
-    }
 }

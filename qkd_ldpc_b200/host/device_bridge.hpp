@@ -30,7 +30,4 @@ namespace qkd_b200
     int usable_devices();
 
     qlb_decode_params params_from_cfg(size_t max_iterations, double threshold);
-
-    // bit packing in the C-ABI's convention
-    void pack_bits(const int *bits, size_t n, uint32_t *words_out);
 }

@@ -58,7 +58,7 @@ struct R_QBER_params
 
 struct config_data
 {
-    size_t THREADS_NUMBER{};
+    size_t THREADS_NUMBER{}; // required and validated as in the reference; the batch sweep runs on GPU worker threads and does not read it
     size_t TRIALS_NUMBER{};
     size_t SIMULATION_SEED{};
     bool INTERACTIVE_MODE{};
@@ -79,8 +79,6 @@ struct config_data
     size_t DEVICE_BATCH_FRAMES = 32768; // "device_batch_frames": most frames per launch handed to one GPU (the on-device key generator needs
                                         // >= 32 k trials in flight to reach its 2.2 M frames/s: 4 096 -> 0.67 M, 16 384 -> 1.83 M; scripts/gen_timing2.py)
     bool DEVICE_FORCE_ALLREDUCE = false; // "device_force_allreduce": run the statistics all-reduce through NCCL even on one GPU (tests)
-    bool DEVICE_GENERATE_KEYS = true;  // "device_generate_keys": draw Alice/Bob on the GPU from the trial seeds (bit-exact with
-                                       // generate_random_bit_array / introduce_errors); false = host threads generate
 };
 
 extern config_data CFG;

@@ -135,12 +135,11 @@ def test_cpp_no_gpu_fails_loudly(sim, tmp_path, lib):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("device_keys", [True, False])
-def test_sweep_csv_equals_reference_north_star(sim, tmp_path, device_keys):
+def test_sweep_csv_equals_reference_north_star(sim, tmp_path):
     """config.json -> CSV on the N=10240 code, 64 trials x 9 QBER points: byte-identical to the CSV written by the
     reference's own main() (tests/golden/sweep_n10240_t64_seed777.csv), fp64 messages; keys drawn on the GPU from the
-    trial seeds (default) or by host threads."""
-    d = make_dir(tmp_path, base_cfg(device_generate_keys=device_keys), NS, False)
+    trial seeds."""
+    d = make_dir(tmp_path, base_cfg(), NS, False)
     run(sim, d)
     out = sorted((d / "results").glob("ldpc*.csv"))
     assert len(out) == 1 and out[0].name == "ldpc(trial_num=64,max_sum_prod_iters=100,seed=777).csv"
