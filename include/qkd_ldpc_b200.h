@@ -14,7 +14,8 @@
  *   - a key / syndrome bit is 0 or 1; "unpacked" arrays hold one 32-bit int per bit
  *     (src/array_and_matrix_operations.hpp:39-40); "packed" arrays hold 32 bits per uint32_t word,
  *     bit i of a frame in word i/32 at bit position i%32, frames padded to whole words
- *     (row stride qlb_code_words_n() / qlb_code_words_m() words);
+ *     (row stride qlb_code_words_n() / qlb_code_words_m() words); the padding bits of a packed input
+ *     are ignored, and those of a packed output are zero;
  *   - LLR sign: positive means bit 0 (src/qkd_ldpc_algorithm.cpp:259-266,401-405);
  *   - node indices are 0-based (src/array_and_matrix_operations.cpp:255,276);
  *   - all host buffers are owned by the caller; the library owns device scratch inside a context.
@@ -132,6 +133,13 @@ int qlb_ctx_device(const qlb_ctx *ctx);
 int qlb_ctx_sm_count(const qlb_ctx *ctx);
 /* The context's CUDA stream (a cudaStream_t) for callers that time or order work with their own events. */
 void *qlb_ctx_stream(const qlb_ctx *ctx);
+/* Which decoder the context's last decode launched, written by the launcher itself (empty before the first decode):
+ *   "generic f64|f64fused|f32|f32fast tier=T shape=S threads=K"       the generic kernel (storage tier, unrolled check shape)
+ *   "resident_f64[fused] bw=B threads=K smem_slots=X/S"             the SM-resident fp64 kernel (X of S message slots in shared memory)
+ *   "resident_f32[fast] bw=B threads=K"                             the SM-resident fp32 kernel
+ *   "stream_f32|f64 vec=V bw=B|any bundle=B waves=W repack=0|1"     the streaming decoder
+ * The string is owned by the context and valid until its next decode. */
+const char *qlb_ctx_last_decoder(const qlb_ctx *ctx);
 int qlb_ctx_synchronize(qlb_ctx *ctx);
 /* Decode-kernel launches and executed frame-iterations since the context was created / last reset. */
 int qlb_ctx_counters(qlb_ctx *ctx, uint64_t *kernel_launches, uint64_t *frame_iterations, int reset);

@@ -25,7 +25,7 @@ EXPORTS = [
     "qlb_code_create", "qlb_code_destroy", "qlb_code_n", "qlb_code_m", "qlb_code_edges", "qlb_code_words_n",
     "qlb_code_words_m", "qlb_code_max_bit_weight", "qlb_code_max_check_weight", "qlb_code_slots", "qlb_code_layout",
     "qlb_code_gather_wavefronts",
-    "qlb_ctx_create", "qlb_ctx_destroy", "qlb_ctx_device", "qlb_ctx_sm_count", "qlb_ctx_stream", "qlb_ctx_synchronize",
+    "qlb_ctx_create", "qlb_ctx_destroy", "qlb_ctx_device", "qlb_ctx_sm_count", "qlb_ctx_stream", "qlb_ctx_last_decoder", "qlb_ctx_synchronize",
     "qlb_ctx_counters", "qlb_ctx_timer_start", "qlb_ctx_timer_stop",
     "qlb_syndrome_batch", "qlb_syndrome_batch_packed", "qlb_sum_product_batch", "qlb_sum_product_trace",
     "qlb_reconcile_batch", "qlb_reconcile_batch_packed", "qlb_reconcile_device", "qlb_stats_allreduce", "qlb_stats_comm_prepare",
@@ -86,6 +86,8 @@ def load_library(path: Path | None = None) -> C.CDLL:
     lib.qlb_ctx_sm_count.argtypes = [vp]
     lib.qlb_ctx_stream.argtypes = [vp]
     lib.qlb_ctx_stream.restype = vp
+    lib.qlb_ctx_last_decoder.argtypes = [vp]
+    lib.qlb_ctx_last_decoder.restype = C.c_char_p
     lib.qlb_ctx_synchronize.argtypes = [vp]
     lib.qlb_ctx_counters.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]
     lib.qlb_ctx_timer_start.argtypes = [vp]
@@ -212,6 +214,11 @@ class Context:
     @property
     def stream(self) -> int:
         return int(self.lib.qlb_ctx_stream(self.handle) or 0)
+
+    @property
+    def last_decoder(self) -> str:
+        """The decoder the last decode on this context launched (qlb_ctx_last_decoder)."""
+        return self.lib.qlb_ctx_last_decoder(self.handle).decode()
 
     def synchronize(self):
         _check(self.lib, self.lib.qlb_ctx_synchronize(self.handle))

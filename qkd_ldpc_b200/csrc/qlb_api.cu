@@ -211,6 +211,9 @@ namespace
         QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
         args.queue = ctx->d_counters;
         args.iter_total = ctx->d_counters + 1;
+        const char *rule = std::is_same<Math, MathF64>::value ? "f64" : std::is_same<Math, MathF64Fused>::value ? "f64fused"
+                         : std::is_same<Math, MathF32Fast>::value ? "f32fast" : "f32";
+        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "generic %s tier=%d shape=%d threads=%d", rule, kTier, kShapeW, kThreads);
         kern<<<(unsigned)grid, kThreads, cv.total_smem, ctx->stream>>>(args);
         QLB_CUDA(cudaGetLastError());
         ++ctx->launches;
@@ -461,6 +464,7 @@ extern "C"
     int qlb_ctx_device(const qlb_ctx *ctx) { return ctx ? ctx->device : -1; }
     int qlb_ctx_sm_count(const qlb_ctx *ctx) { return ctx ? ctx->sm_count : 0; }
     void *qlb_ctx_stream(const qlb_ctx *ctx) { return ctx ? (void *)ctx->stream : nullptr; }
+    const char *qlb_ctx_last_decoder(const qlb_ctx *ctx) { return ctx ? ctx->last_decoder : ""; }
     int qlb_ctx_synchronize(qlb_ctx *ctx)
     {
         if (!ctx)

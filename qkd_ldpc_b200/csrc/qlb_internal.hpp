@@ -77,6 +77,7 @@ struct qlb_ctx
     qlb::DevBuf scratch, in_a, in_b, in_q, in_llr, in_syn, out_it, out_res, out_dec, out_syn, gen_perm, gen_seeds;
     std::vector<double> host_logp;
     std::vector<uint32_t> host_pack_a, host_pack_b, host_pack_out;
+    char last_decoder[128] = {}; // written by each decode launcher just before it launches (qlb_ctx_last_decoder)
 };
 
 namespace qlb

@@ -772,8 +772,10 @@ namespace qlb
                 const uint32_t zw = s_z[w];
                 if (args.decoded)
                     args.decoded[f * words_n + w] = zw;
+                // arrays_equal(alice, decoded) (:433) over the n key bits: the padding bits of Alice's last word are not part of the key
+                const uint32_t key_mask = (w == words_n - 1 && (n & 31)) ? (1u << (n & 31)) - 1u : 0xFFFFFFFFu;
                 if (kReconcile)
-                    differs |= (zw != s_alice[w]); // arrays_equal(alice, decoded) (:433)
+                    differs |= ((zw ^ s_alice[w]) & key_mask) != 0;
             }
             if (kReconcile && args.syndrome_out)
                 for (int w = tid; w < words_m; w += kThreads)

@@ -26,6 +26,8 @@ namespace
         QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
         args.queue = ctx->d_counters;
         args.iter_total = ctx->d_counters + 1;
+        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "resident_f32%s bw=%d threads=%d",
+                      std::is_same<Rule, RuleF32Fast>::value ? "fast" : "", kBW, kThreads);
         kern<<<(unsigned)grid, kThreads, smem, ctx->stream>>>(args);
         QLB_CUDA(cudaGetLastError());
         ++ctx->launches;

@@ -52,6 +52,8 @@ namespace
         QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
         args.queue = ctx->d_counters;
         args.iter_total = ctx->d_counters + 1;
+        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "resident_f64%s bw=%d threads=%d smem_slots=%u/%d",
+                      std::is_same<Math, MathF64Fused>::value ? "fused" : "", kBW, kThreads, c.r64_smem_slots, c.slots);
         kern<<<(unsigned)grid, kThreads, smem, ctx->stream>>>(args);
         QLB_CUDA(cudaGetLastError());
         ++ctx->launches;

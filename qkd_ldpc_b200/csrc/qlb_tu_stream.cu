@@ -80,6 +80,9 @@ namespace
             std::fprintf(stderr, "[qlb] stream split VEC=%d: %lld groups of %lld frames, bundles of %d, %lld wave(s) of <= %lld groups, %zu B per bundle; check grid %u (%d/SM), bit grid %u (%d/SM)\n",
                          VEC, groups, G, B, waves, per_wave, per_bundle, grid_check, occ_check, grid_bit, occ_bit);
 #endif
+        const char bw[2] = {kBW ? (char)('0' + kBW) : '\0', '\0'};
+        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "stream_%s vec=%d bw=%s bundle=%d waves=%lld repack=%d",
+                      sizeof(Real) == 4 ? "f32" : "f64", VEC, kBW ? bw : "any", B, waves, (int)repack_on);
         for (long long w = 0; w < waves; ++w)
         {
             st.group0 = w * per_wave;
