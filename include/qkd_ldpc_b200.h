@@ -60,8 +60,10 @@ enum {
      * by the SM-resident fp64 kernel and by the generic kernel (checks wider than its unrolled shapes keep the literal order).
      * Per-frame outcomes validated against the reference in profiles/parity_r01.md and on the exhaustive small-code fixtures. */
     QLB_FLAG_F64_FUSED_RATIO = 2,
-    /* test hook, bits 8..11 = 1 + storage tier (0 shared memory, 1 L2 scratch for messages, 2 all global): run the generic
-     * kernel in that tier instead of the fastest eligible one; ignored when the tier does not fit */
+    /* test hook, bits 8..11 = 1 + hook (0: no hook). Hooks 0 / 1 / 2 run the generic kernel in that storage tier (0 shared
+     * memory, 1 L2 scratch for messages, 2 all global) instead of the fastest eligible decoder; a tier faster than the fastest
+     * the code fits in is ignored. Hook 3 runs the streaming decoder, or fails with QLB_ERR_UNSUPPORTED when it does not take
+     * the code. Hooks above 3 are rejected with QLB_ERR_INVALID. */
     QLB_FLAG_TEST_TIER_SHIFT = 8
 };
 

@@ -38,43 +38,47 @@ def _newer(target: Path, sources) -> bool:
     return all(Path(s).stat().st_mtime <= t for s in sources)
 
 
-def _run(cmd, log_name):
+def _run(cmd, log: Path):
     proc = subprocess.run([str(c) for c in cmd], capture_output=True, text=True)
-    (LIB_DIR / log_name).write_text(proc.stdout + proc.stderr)
+    log.write_text(proc.stdout + proc.stderr)
     if proc.returncode != 0:
         sys.stderr.write(proc.stdout + proc.stderr)
         raise RuntimeError(f"build failed: {' '.join(str(c) for c in cmd)}")
 
 
-TRANSLATION_UNITS = ["qlb_api.cu", "qlb_tu_resident_f32.cu", "qlb_tu_stream.cu", "qlb_tu_resident_f64.cu"]
+TRANSLATION_UNITS = ["qlb_api.cu", "qlb_tu_generic.cu", "qlb_tu_resident_f32.cu", "qlb_tu_stream.cu", "qlb_tu_resident_f64.cu"]
 
 
-def build_library(force: bool = False, verbose_ptxas: bool = True) -> Path:
-    """One object per kernel family, compiled in parallel, linked into libqkdldpc_b200.so."""
+def build_library(force: bool = False, verbose_ptxas: bool = True, out: Path = LIB_PATH, extra_flags=()) -> Path:
+    """One object per translation unit, compiled in parallel, linked into `out` (default: libqkdldpc_b200.so).
+    `extra_flags`: more nvcc flags, e.g. the -D knobs of a variant library; a library other than the default keeps its objects
+    and logs in a directory of its own beside it."""
     from concurrent.futures import ThreadPoolExecutor
-    LIB_DIR.mkdir(exist_ok=True)
-    obj_dir = LIB_DIR / "obj"
-    obj_dir.mkdir(exist_ok=True)
+    out = Path(out)
+    work = LIB_DIR if out == LIB_PATH else out.parent / (out.stem + "_build")
+    obj_dir = work / "obj"
+    obj_dir.mkdir(parents=True, exist_ok=True)
     headers = sorted(CSRC.glob("*.cuh")) + sorted(CSRC.glob("*.hpp")) + [ROOT / "include" / "qkd_ldpc_b200.h"]
     sources = [CSRC / tu for tu in TRANSLATION_UNITS]
-    if not force and _newer(LIB_PATH, sources + headers):
-        return LIB_PATH
+    if not force and _newer(out, sources + headers):
+        return out
+    flags = [*NVCC_FLAGS, *extra_flags]
 
     def compile_tu(src: Path) -> Path:
         obj = obj_dir / (src.stem + ".o")
         if force or not _newer(obj, [src] + headers):
-            cmd = [NVCC, *NVCC_FLAGS, "-c", "-o", obj, src]
+            cmd = [NVCC, *flags, "-c", "-o", obj, src]
             if verbose_ptxas:
                 cmd += ["-Xptxas", "-v"]
-            _run(cmd, f"build_{src.stem}.log")
+            _run(cmd, work / f"build_{src.stem}.log")
         return obj
 
     with ThreadPoolExecutor(max_workers=len(sources)) as pool:
         objs = list(pool.map(compile_tu, sources))
-    _run([NVCC, *NVCC_FLAGS, "-shared", "-o", LIB_PATH, *objs, "-ldl"], "build_link.log")
-    (LIB_DIR / "build_lib.log").write_text("".join((LIB_DIR / f"build_{src.stem}.log").read_text() for src in sources
-                                                   if (LIB_DIR / f"build_{src.stem}.log").exists()))
-    return LIB_PATH
+    _run([NVCC, *flags, "-shared", "-o", out, *objs, "-ldl"], work / "build_link.log")
+    (work / "build_lib.log").write_text("".join((work / f"build_{src.stem}.log").read_text() for src in sources
+                                                if (work / f"build_{src.stem}.log").exists()))
+    return out
 
 
 def build_host(force: bool = False) -> Path | None:
@@ -88,7 +92,7 @@ def build_host(force: bool = False) -> Path | None:
         return SIM_PATH
     cmd = [HOST_CXX, "-std=c++20", "-O2", "-Wall", "-pthread", f"-I{ROOT / 'include'}", f"-I{HOST}", "-o", SIM_PATH, *srcs,
            f"-L{LIB_DIR}", "-lqkdldpc_b200", f"-Wl,-rpath,{LIB_DIR}", "-Wl,-rpath,$ORIGIN/../lib", "-ldl"]
-    _run(cmd, "build_host.log")
+    _run(cmd, LIB_DIR / "build_host.log")
     return SIM_PATH
 
 

@@ -131,7 +131,7 @@ def make_params(precision=64, max_iterations=100, threshold=100.0, enable_thresh
     else:
         flags = 0
     if tier is not None:
-        flags |= (int(tier) + 1) << 8  # QLB_FLAG_TEST_TIER: force a slower storage tier
+        flags |= (int(tier) + 1) << 8  # QLB_FLAG_TEST_TIER_SHIFT hook: 0 ... 2 a generic kernel storage tier, 3 the streaming decoder
     return DecodeParams(int(precision), int(max_iterations), int(bool(enable_threshold)), flags, float(threshold),
                         int(stream_max_bundles), int(bool(stream_no_repack)), int(block_threads), 0)
 

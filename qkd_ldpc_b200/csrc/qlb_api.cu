@@ -180,115 +180,9 @@ namespace
             return fail(QLB_ERR_INVALID, "QLB_FLAG_F64_FUSED_RATIO requires fp64 precision");
         if (p->stream_max_bundles < 0 || p->block_threads < 0 || p->reserved != 0)
             return fail(QLB_ERR_INVALID, "qlb_decode_params: negative execution knob or non-zero reserved field");
+        if (((p->flags >> QLB_FLAG_TEST_TIER_SHIFT) & 0xF) > 4)
+            return fail(QLB_ERR_INVALID, "qlb_decode_params.flags: the test hook (bits 8..11) must be 0 (none) or 1 + hook, hook 0 ... 3");
         return QLB_OK;
-    }
-
-    // ---- kernel selection ---------------------------------------------------------------------------------------
-    template <typename Math, int kTier, bool kReconcile, int kShapeW, int kThreads>
-    int launch_one(qlb_ctx *ctx, DecodeArgs &args)
-    {
-        typedef typename Math::real Real;
-        auto kern = decode_kernel<Math, kTier, kReconcile, kShapeW, kThreads>;
-        const Carve cv = make_carve<Real, kTier>(args.code.n, args.code.m, args.code.slots, args.code.max_bit_w);
-        QLB_CUDA(allow_full_dynamic_smem(ctx, kern));
-        int per_sm = 0;
-        QLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, cv.total_smem));
-        if (per_sm < 1)
-            return fail(QLB_ERR_UNSUPPORTED, "decode kernel does not fit on an SM for this code");
-        long long grid = (long long)ctx->sm_count * per_sm;
-        if (grid > args.n_frames)
-            grid = args.n_frames;
-        if (cv.total_scratch)
-        {
-            QLB_CUDA(ctx->scratch.reserve((size_t)grid * cv.total_scratch));
-            args.scratch = static_cast<unsigned char *>(ctx->scratch.p);
-            args.scratch_stride = cv.total_scratch;
-        }
-#ifdef QLB_DEBUG_LAUNCH
-            std::fprintf(stderr, "[qlb] decode_kernel tier=%d reconcile=%d shapeW=%d threads=%d: %d CTA/SM, grid=%lld, smem=%zu B, scratch=%zu B/CTA\n",
-                         kTier, (int)kReconcile, kShapeW, kThreads, per_sm, grid, cv.total_smem, cv.total_scratch);
-#endif
-        QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
-        args.queue = ctx->d_counters;
-        args.iter_total = ctx->d_counters + 1;
-        const char *rule = std::is_same<Math, MathF64>::value ? "f64" : std::is_same<Math, MathF64Fused>::value ? "f64fused"
-                         : std::is_same<Math, MathF32Fast>::value ? "f32fast" : "f32";
-        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "generic %s tier=%d shape=%d threads=%d", rule, kTier, kShapeW, kThreads);
-        kern<<<(unsigned)grid, kThreads, cv.total_smem, ctx->stream>>>(args);
-        QLB_CUDA(cudaGetLastError());
-        ++ctx->launches;
-        return QLB_OK;
-    }
-
-    template <typename Math, int kTier, bool kReconcile, int kThreads>
-    int launch_shape(qlb_ctx *ctx, DecodeArgs &args)
-    {
-        const int cw = args.code.max_check_w, bw = args.code.max_bit_w;
-        if constexpr (kTier != kTierGlobal) // register-tile variants exist for the shared-memory tiers only
-        {
-            if (bw <= 4 && cw <= 8)
-                return launch_one<Math, kTier, kReconcile, 8, kThreads>(ctx, args);
-            if (bw <= 4 && cw <= 16)
-                return launch_one<Math, kTier, kReconcile, 16, kThreads>(ctx, args);
-        }
-        return launch_one<Math, kTier, kReconcile, 0, kThreads>(ctx, args);
-    }
-
-    template <typename Math, bool kReconcile>
-    int launch_tier(qlb_ctx *ctx, DecodeArgs &args, int forced_tier)
-    {
-        typedef typename Math::real Real;
-        const CodeDev &c = args.code;
-        const bool idx16 = c.slots < 65535 && c.bit_slots16 != nullptr;
-        const size_t all = make_carve<Real, kTierSmemAll>(c.n, c.m, c.slots, c.max_bit_w).total_smem;
-        const size_t idx = make_carve<Real, kTierSmemIdx>(c.n, c.m, c.slots, c.max_bit_w).total_smem;
-        int tier = kTierGlobal;
-        if (idx16 && idx <= (size_t)ctx->smem_optin)
-            tier = kTierSmemIdx;
-        if (idx16 && sizeof(Real) == 4 && all <= (size_t)ctx->smem_optin)
-            tier = kTierSmemAll;
-        if (forced_tier >= 0 && forced_tier >= tier)
-            tier = forced_tier; // tests may force a slower tier, never one that does not fit
-        if constexpr (sizeof(Real) == 4) // fp64 messages never fit a whole frame in shared memory
-        {
-            if (tier == kTierSmemAll)
-                return launch_shape<Math, kTierSmemAll, kReconcile, 1024>(ctx, args);
-        }
-        if (tier == kTierSmemIdx)
-            return launch_shape<Math, kTierSmemIdx, kReconcile, 512>(ctx, args);
-        return launch_shape<Math, kTierGlobal, kReconcile, 512>(ctx, args);
-    }
-
-    template <bool kReconcile>
-    int launch_decode(qlb_ctx *ctx, const qlb_decode_params *p, DecodeArgs &args)
-    {
-        args.max_it = p->max_iterations;
-        args.enable_thr = p->enable_threshold;
-        args.thr = p->threshold;
-        args.cap_f32 = p->enable_threshold ? (float)p->threshold : INFINITY;
-        args.stream_max_bundles = p->stream_max_bundles;
-        args.stream_no_repack = p->stream_no_repack;
-        args.block_threads = p->block_threads;
-        const int forced = (p->flags >> 8) & 0xF ? ((p->flags >> 8) & 0xF) - 1 : -1; // bits 8..11: test hook, tier+1
-        const bool fast = (p->flags & QLB_FLAG_F32_FAST_MATH) != 0;
-        if (p->precision == QLB_PRECISION_F32 && forced < 0 && resident_f32_eligible(ctx, args.code))
-            return launch_resident_f32(ctx, args, kReconcile, fast);
-        // codes too large for one SM's shared memory: frame-interleaved streaming through HBM (test hook: tier 3 forces it)
-        if (p->precision == QLB_PRECISION_F32 && (forced < 0 || forced == 3) && stream_eligible(args.code))
-            return launch_stream_f32(ctx, args, kReconcile, fast);
-        if (p->precision == QLB_PRECISION_F64 && forced < 0 && resident_f64_eligible(ctx, args.code))
-            return launch_resident_f64(ctx, args, kReconcile, (p->flags & QLB_FLAG_F64_FUSED_RATIO) != 0);
-        // fp64 at block lengths whose indices do not fit the generic kernel's shared-memory tiers: the fp64 streaming decoder
-        if (p->precision == QLB_PRECISION_F64 && (forced == 3 || (forced < 0 && args.code.slots >= 65535)) && stream_eligible(args.code))
-            return launch_stream_f64(ctx, args, kReconcile, (p->flags & QLB_FLAG_F64_FUSED_RATIO) != 0);
-        if (forced == 3)
-            return fail(QLB_ERR_UNSUPPORTED, "the streaming kernel does not handle this code / precision");
-        if (p->precision == QLB_PRECISION_F64)
-            return (p->flags & QLB_FLAG_F64_FUSED_RATIO) ? launch_tier<MathF64Fused, kReconcile>(ctx, args, forced)
-                                                         : launch_tier<MathF64, kReconcile>(ctx, args, forced);
-        if (fast)
-            return launch_tier<MathF32Fast, kReconcile>(ctx, args, forced);
-        return launch_tier<MathF32, kReconcile>(ctx, args, forced);
     }
 
     int launch_syndrome(qlb_ctx *ctx, const CodeDev &dev, long long n_frames, const uint32_t *d_bits, uint32_t *d_out)
@@ -581,7 +475,7 @@ extern "C"
         args.result = d_result_out;
         args.decoded = d_decoded_packed_out;
         args.syndrome_out = d_syndrome_packed_out;
-        return launch_decode<true>(ctx, params, args);
+        return launch_decode(ctx, *params, true, args);
     }
 
     int qlb_reconcile_batch_packed(qlb_ctx *ctx, const qlb_code *code, const qlb_decode_params *params, int64_t n_frames,
@@ -710,7 +604,7 @@ extern "C"
         args.iterations = (uint32_t *)ctx->out_it.p;
         args.result = (uint8_t *)ctx->out_res.p;
         args.decoded = (uint32_t *)ctx->out_dec.p;
-        if ((rc = launch_decode<false>(ctx, params, args)))
+        if ((rc = launch_decode(ctx, *params, false, args)))
             return rc;
         QLB_CUDA(cudaMemcpyAsync(iterations_out, ctx->out_it.p, (size_t)n_frames * 4, cudaMemcpyDeviceToHost, ctx->stream));
         QLB_CUDA(cudaMemcpyAsync(result_out, ctx->out_res.p, (size_t)n_frames, cudaMemcpyDeviceToHost, ctx->stream));

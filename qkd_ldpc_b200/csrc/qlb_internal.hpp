@@ -1,15 +1,19 @@
 // Internal declarations shared by the translation units of libqkdldpc_b200.so (not part of the C-ABI).
-// The library is split into one TU per kernel family so that they compile in parallel:
-//   qlb_api.cu            C-ABI, code/context management, generic decode_kernel, syndrome, key generator
-//   qlb_tu_resident_f32.cu / qlb_tu_stream_f32.cu / qlb_tu_resident_f64.cu   the specialised decoders + their launchers
+// The library is split into TUs that compile in parallel: qlb_api.cu (C-ABI, code/context management, syndrome, key generator,
+// trace) and one per decoder family, with its admission predicate and its launcher: qlb_tu_generic.cu, qlb_tu_resident_f32.cu,
+// qlb_tu_resident_f64.cu, qlb_tu_stream.cu. route_decode, below, chooses the family of a batch.
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <map>
 #include <string>
+#include <tuple>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/qkd_ldpc_b200.h"
@@ -95,49 +99,112 @@ namespace qlb
         return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - (int)fa.sharedSizeBytes);
     }
 
-    // Block size (multiple of 32, in [max/2, max]) for the thread-per-node kernels. Every thread walks the bits with stride T and each
-    // weight segment of the sorted checks with stride T, and the block waits for the slowest thread, so T is chosen to keep the
-    // last round of each walk as full as possible (`check_share`: the check walk's share of an iteration); among equally balanced
-    // sizes the smaller block measured slightly faster (B200, N=10240: 768 > 896 > 1024 threads by 2 %). Both walks must stay within the 32 per-thread rounds the kernels park bits for.
-    // `min_threads`: the fp64 kernel is latency-bound (dependent DFMA chains, L2 index loads) and wants warps more than balance:
-    // measured on B200, N=10240, fused rule: 384 / 512 / 640 / 768 threads = 3.08 / 3.46 / 3.61 / 3.87 M frame-iterations/s
-    // (`size_bias` > 0: among equally balanced sizes the larger block).
-    inline int balanced_block_size(const CodeDev &c, int max_threads, double check_share, int min_threads = 0, double size_bias = -0.02)
+    enum class Rule { F64, F64Fused, F32, F32Fast }; // the precision and its cheaper check rule (QLB_FLAG_F32_FAST_MATH / F64_FUSED_RATIO)
+    enum class Family { ResidentF32, ResidentF64, Stream, Generic };
+    struct Route // the decoder that takes a batch, and how it runs
     {
-        int best = 0;
-        double best_score = -1.;
-        if (min_threads <= 0)
-            min_threads = max_threads / 2;
-        for (int t = max_threads; t >= min_threads && t >= 32; t -= 32)
-        {
-            long long check_rounds = 0;
-            for (int w = c.max_check_w; w >= 0; --w)
-            {
-                const long long lo = (w < c.max_check_w) ? c.cnt[w] : 0, hi = (w > 0) ? c.cnt[w - 1] : c.m;
-                check_rounds += (hi - lo + t - 1) / t;
-            }
-            const long long bit_rounds = (c.n + t - 1) / t;
-            if (check_rounds > 32 || bit_rounds > 32)
-                break;
-            const double ec = (double)c.m / t / (double)check_rounds, eb = (double)c.n / t / (double)bit_rounds;
-            const double score = (check_share * ec + (1. - check_share) * eb) * (1. + size_bias * t / max_threads);
-            if (score > best_score + 1e-12)
-            {
-                best_score = score;
-                best = t;
-            }
-        }
-        return best; // 0: no admissible block size
-    }
+        Family family;
+        Rule rule;
+        bool reconcile; // reconcile mode (keys and log prior) or sum-product mode (LLRs and syndrome)
+        Tier tier;      // generic kernel: storage tier
+        int32_t stream_max_bundles, stream_no_repack, block_threads; // qlb_decode_params' execution knobs
+    };
 
-    // launchers of the specialised decoders (each in its own TU); `fast`: the SFU check rule
+    // One TU per decoder family: admission predicate (fp64 resident: the code has group tables) and launcher.
     bool resident_f32_eligible(const qlb_ctx *ctx, const CodeDev &c);
-    int launch_resident_f32(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fast);
-    bool stream_eligible(const CodeDev &c);
-    int launch_stream_f32(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fast);
-    int launch_stream_f64(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fused); // `fused`: the fused-ratio check rule
-    bool resident_f64_eligible(const qlb_ctx *ctx, const CodeDev &c);
+    int launch_resident_f32(qlb_ctx *ctx, DecodeArgs &args, const Route &r);
     bool resident64_build_tables(const qlb_ctx *ctx, const CodeDev &c, const uint32_t *bit_slots, std::vector<uint32_t> &check_groups,
                                  std::vector<uint16_t> &bit_groups, uint32_t &smem_slots);
-    int launch_resident_f64(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fused);
+    int launch_resident_f64(qlb_ctx *ctx, DecodeArgs &args, const Route &r);
+    bool stream_eligible(const CodeDev &c);
+    int launch_stream(qlb_ctx *ctx, DecodeArgs &args, const Route &r);
+    Tier generic_tier(const qlb_ctx *ctx, const CodeDev &c, bool fp32); // the fastest storage tier the code fits in
+    int launch_generic(qlb_ctx *ctx, DecodeArgs &args, const Route &r);
+
+    // The node arithmetic (qlb_kernels.cuh) of each rule in the generic kernel and the fp64 decoders.
+    template <Rule kRule> using MathOf = std::tuple_element_t<(int)kRule, std::tuple<MathF64, MathF64Fused, MathF32, MathF32Fast>>;
+
+    // Calls f(rule, reconcile) with the route's rule and mode as std::integral_constant<Rule, ...> and std::bool_constant: template
+    // arguments for a launcher. Only the listed rules, those the family implements (route_decode picks no other), are instantiated.
+    template <Rule kRule, Rule... kMore, typename F>
+    int with_rule(const Route &r, F &&f)
+    {
+        if constexpr (sizeof...(kMore) > 0)
+            if (r.rule != kRule)
+                return with_rule<kMore...>(r, f);
+        if (r.reconcile)
+            return f(std::integral_constant<Rule, kRule>{}, std::true_type{});
+        return f(std::integral_constant<Rule, kRule>{}, std::false_type{});
+    }
+
+    // The launch of a persistent decoder: min(SMs x ctas_per_sm, frames) CTAs, each taking frames from the queue counter until
+    // none is left. `scratch`: global scratch bytes per CTA (0: none). `decoder`: what qlb_ctx_last_decoder reports.
+    template <typename Kernel>
+    int launch_persistent(qlb_ctx *ctx, DecodeArgs &args, Kernel kern, int threads, size_t smem, int ctas_per_sm, size_t scratch,
+                          const char *decoder)
+    {
+        QLB_CUDA(allow_full_dynamic_smem(ctx, kern));
+        const long long grid = std::min<long long>((long long)ctx->sm_count * ctas_per_sm, args.n_frames);
+        if (scratch)
+        {
+            QLB_CUDA(ctx->scratch.reserve((size_t)grid * scratch));
+            args.scratch = static_cast<unsigned char *>(ctx->scratch.p);
+            args.scratch_stride = scratch;
+        }
+#ifdef QLB_DEBUG_LAUNCH
+        std::fprintf(stderr, "[qlb] %s: %d CTA/SM, grid=%lld, smem=%zu B, scratch=%zu B/CTA\n", decoder, ctas_per_sm, grid, smem, scratch);
+#endif
+        QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
+        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "%s", decoder);
+        kern<<<(unsigned)grid, threads, smem, ctx->stream>>>(args);
+        QLB_CUDA(cudaGetLastError());
+        ++ctx->launches;
+        return QLB_OK;
+    }
+
+    // The decoder of a batch of checked parameters: the order of the tests is the whole policy.
+    inline int route_decode(const qlb_ctx *ctx, const CodeDev &c, const qlb_decode_params &p, bool reconcile, Route &out)
+    {
+        const bool fp32 = p.precision == QLB_PRECISION_F32;
+        // test hook (QLB_FLAG_TEST_TIER_SHIFT; check_params admits 0 ... 3): -1 none, 0 ... 2 the generic kernel in that storage
+        // tier or a slower one, 3 the streaming decoder
+        const int hook = ((p.flags >> QLB_FLAG_TEST_TIER_SHIFT) & 0xF) - 1;
+        Rule rule = fp32 ? Rule::F32 : Rule::F64;
+        if (p.flags & (fp32 ? QLB_FLAG_F32_FAST_MATH : QLB_FLAG_F64_FUSED_RATIO)) // the precision's cheaper check rule
+            rule = fp32 ? Rule::F32Fast : Rule::F64Fused;
+        out = Route{Family::Generic, rule, reconcile, kTierGlobal, p.stream_max_bundles, p.stream_no_repack, p.block_threads};
+        if (hook < 0 && (fp32 ? resident_f32_eligible(ctx, c) : c.r64_check_group_table != nullptr))
+            out.family = fp32 ? Family::ResidentF32 : Family::ResidentF64;
+        // frame-interleaved streaming through HBM: in fp32 every code the resident kernel rejects; in fp64 the block lengths whose
+        // slot indices do not fit the generic kernel's shared-memory tiers
+        else if ((hook == 3 || (hook < 0 && (fp32 || c.slots >= 65535))) && stream_eligible(c))
+            out.family = Family::Stream;
+        else if (hook == 3)
+            return fail(QLB_ERR_UNSUPPORTED, "the streaming kernel does not handle this code / precision");
+        else // tests may force a slower tier, never one that does not fit
+            out.tier = (Tier)std::max<int>(generic_tier(ctx, c, fp32), hook);
+        return QLB_OK;
+    }
+
+    // The decode of a batch: its route, the arguments every decoder reads, the launch.
+    inline int launch_decode(qlb_ctx *ctx, const qlb_decode_params &p, bool reconcile, DecodeArgs &args)
+    {
+        Route r;
+        if (const int rc = route_decode(ctx, args.code, p, reconcile, r))
+            return rc;
+        args.queue = ctx->d_counters;
+        args.iter_total = ctx->d_counters + 1;
+        args.max_it = p.max_iterations;
+        args.enable_thr = p.enable_threshold;
+        args.thr = p.threshold;
+        args.cap_f32 = p.enable_threshold ? (float)p.threshold : INFINITY;
+        switch (r.family)
+        {
+        case Family::ResidentF32: return launch_resident_f32(ctx, args, r);
+        case Family::ResidentF64: return launch_resident_f64(ctx, args, r);
+        case Family::Stream: return launch_stream(ctx, args, r);
+        case Family::Generic: return launch_generic(ctx, args, r);
+        }
+        return fail(QLB_ERR_INVALID, "decode route: unknown decoder family");
+    }
 }

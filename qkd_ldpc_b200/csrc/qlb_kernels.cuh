@@ -99,8 +99,6 @@ namespace qlb
         unsigned long long *iter_total; // sum of executed iterations
         unsigned char *scratch;         // per-CTA global scratch (tiers 1, 2)
         size_t scratch_stride;
-        // host-side launch knobs (qlb_decode_params; not read by kernels)
-        int32_t stream_max_bundles, stream_no_repack, block_threads;
     };
 
     // ------------------------------------------------------------------------------------------------------------

@@ -1,51 +1,57 @@
 #include "qlb_internal.hpp"
-#include <algorithm>
 using namespace qlb;
 #include "qlb_resident_f32.cuh"
 
 namespace
 {
-    // The specialised fp32 kernel (qlb_resident_f32.cuh): whole frame in shared memory, uniform bit weight.
-    template <typename Rule, bool kReconcile, int kBW>
-    int launch_resident(qlb_ctx *ctx, DecodeArgs &args)
+    // Block size (multiple of 32, in [max/2, max]). Every thread walks the bits with stride T and each weight segment of the sorted
+    // checks with stride T, and the block waits for the slowest thread, so T is chosen to keep the last round of each walk as full
+    // as possible (`check_share`: the check walk's share of an iteration); among equally balanced sizes the smaller block measured
+    // slightly faster (B200, N=10240: 768 > 896 > 1024 threads by 2 %). Both walks must stay within the 32 per-thread rounds the kernel parks bits for.
+    int balanced_block_size(const CodeDev &c, int max_threads, double check_share)
     {
-        auto kern = decode_resident_f32_kernel<Rule, kReconcile, kBW, kResidentThreads>;
+        int best = 0;
+        double best_score = -1.;
+        for (int t = max_threads; t >= max_threads / 2 && t >= 32; t -= 32)
+        {
+            long long check_rounds = 0;
+            for (int w = c.max_check_w; w >= 0; --w)
+            {
+                const long long lo = (w < c.max_check_w) ? c.cnt[w] : 0, hi = (w > 0) ? c.cnt[w - 1] : c.m;
+                check_rounds += (hi - lo + t - 1) / t;
+            }
+            const long long bit_rounds = (c.n + t - 1) / t;
+            if (check_rounds > 32 || bit_rounds > 32)
+                break;
+            const double ec = (double)c.m / t / (double)check_rounds, eb = (double)c.n / t / (double)bit_rounds;
+            const double score = (check_share * ec + (1. - check_share) * eb) * (1. - 0.02 * t / max_threads);
+            if (score > best_score + 1e-12)
+            {
+                best_score = score;
+                best = t;
+            }
+        }
+        return best; // 0: no admissible block size
+    }
+
+    // The specialised fp32 kernel (qlb_resident_f32.cuh): whole frame in shared memory, uniform bit weight.
+    template <typename CheckRule, bool kReconcile, int kBW>
+    int launch_resident(qlb_ctx *ctx, DecodeArgs &args, int block_threads)
+    {
+        auto kern = decode_resident_f32_kernel<CheckRule, kReconcile, kBW, kResidentThreads>;
         int kThreads = balanced_block_size(args.code, kResidentThreads, 0.55);
-        if (const int t = args.block_threads / 32 * 32) // qlb_decode_params.block_threads
+        if (const int t = block_threads / 32 * 32) // qlb_decode_params.block_threads
             if (t >= 32 && t <= kResidentThreads && 32 * t >= args.code.n && 32 * t >= args.code.m)
                 kThreads = t;
         const size_t smem = resident_smem_bytes(args.code.n, args.code.m, args.code.slots, kBW);
-        QLB_CUDA(allow_full_dynamic_smem(ctx, kern));
-        long long grid = ctx->sm_count; // one resident CTA per SM
-        if (grid > args.n_frames)
-            grid = args.n_frames;
 #ifdef QLB_BOUNDS_CHECK
         const uint32_t msg_bytes = 4u * (uint32_t)args.code.slots;
         QLB_CUDA(cudaMemcpyToSymbolAsync(g_bounds_msg_bytes, &msg_bytes, 4, 0, cudaMemcpyHostToDevice, ctx->stream));
 #endif
-        QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
-        args.queue = ctx->d_counters;
-        args.iter_total = ctx->d_counters + 1;
-        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "resident_f32%s bw=%d threads=%d",
-                      std::is_same<Rule, RuleF32Fast>::value ? "fast" : "", kBW, kThreads);
-        kern<<<(unsigned)grid, kThreads, smem, ctx->stream>>>(args);
-        QLB_CUDA(cudaGetLastError());
-        ++ctx->launches;
-        return QLB_OK;
+        char name[sizeof(qlb_ctx::last_decoder)];
+        std::snprintf(name, sizeof name, "resident_f32%s bw=%d threads=%d", std::is_same<CheckRule, RuleF32Fast>::value ? "fast" : "", kBW, kThreads);
+        return launch_persistent(ctx, args, kern, kThreads, smem, 1, 0, name); // one resident CTA per SM
     }
-
-    template <typename Rule, bool kReconcile>
-    int launch_resident_bw(qlb_ctx *ctx, DecodeArgs &args)
-    {
-        switch (args.code.uniform_bit_w)
-        {
-        case 2: return launch_resident<Rule, kReconcile, 2>(ctx, args);
-        case 3: return launch_resident<Rule, kReconcile, 3>(ctx, args);
-        case 4: return launch_resident<Rule, kReconcile, 4>(ctx, args);
-        default: return fail(QLB_ERR_UNSUPPORTED, "resident kernel: unsupported bit weight");
-        }
-    }
-
 }
 namespace qlb
 {
@@ -56,10 +62,19 @@ namespace qlb
                resident_smem_bytes(c.n, c.m, c.slots, c.uniform_bit_w) + kResidentStaticSmem <= (size_t)ctx->smem_optin;
     }
 
-    int launch_resident_f32(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fast)
+    int launch_resident_f32(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        if (fast)
-            return reconcile ? launch_resident_bw<RuleF32Fast, true>(ctx, args) : launch_resident_bw<RuleF32Fast, false>(ctx, args);
-        return reconcile ? launch_resident_bw<RuleF32Accurate, true>(ctx, args) : launch_resident_bw<RuleF32Accurate, false>(ctx, args);
+        return with_rule<Rule::F32, Rule::F32Fast>(r, [&](auto rule, auto reconcile) -> int
+        {
+            typedef std::conditional_t<decltype(rule)::value == Rule::F32Fast, RuleF32Fast, RuleF32Accurate> CheckRule;
+            constexpr bool kReconcile = decltype(reconcile)::value;
+            switch (args.code.uniform_bit_w)
+            {
+            case 2: return launch_resident<CheckRule, kReconcile, 2>(ctx, args, r.block_threads);
+            case 3: return launch_resident<CheckRule, kReconcile, 3>(ctx, args, r.block_threads);
+            case 4: return launch_resident<CheckRule, kReconcile, 4>(ctx, args, r.block_threads);
+            default: return fail(QLB_ERR_UNSUPPORTED, "resident kernel: unsupported bit weight");
+            }
+        });
     }
 }

@@ -1,5 +1,4 @@
 #include "qlb_internal.hpp"
-#include <algorithm>
 using namespace qlb;
 #include "qlb_resident_f64.cuh"
 
@@ -19,75 +18,34 @@ namespace
         return (uint32_t)std::min<size_t>(fit, (size_t)c.slots);
     }
 
-    bool resident64_eligible_impl(const qlb_ctx *ctx, const CodeDev &c)
-    {
-        return c.slots < 65535 && c.n < 65536 && c.m < 65536 && c.bit_slots16 && c.col_of_slot16 && c.uniform_bit_w >= 2 && c.uniform_bit_w <= 4 &&
-               c.max_check_w <= kResidentMaxCW && c.n % 32 == 0 && resident64_smem_slots(ctx, c) >= (uint32_t)c.slots / 2;
-    }
-
     template <typename Math, bool kReconcile, int kBW>
-    int launch_resident64(qlb_ctx *ctx, DecodeArgs &args)
+    int launch_resident64(qlb_ctx *ctx, DecodeArgs &args, int block_threads)
     {
         auto kern = decode_resident_f64_kernel<Math, kReconcile, kBW, kResident64Threads>;
         const CodeDev &c = args.code;
-        if (!c.r64_check_group_table || !c.r64_bit_group_table)
-            return fail(QLB_ERR_UNSUPPORTED, "fp64 resident kernel: the code carries no group tables");
         int kThreads = kResident64Threads;
-        if (const int t = args.block_threads / 32 * 32) // qlb_decode_params.block_threads
+        if (const int t = block_threads / 32 * 32) // qlb_decode_params.block_threads
             if (t >= 32 && t <= kResident64Threads)
                 kThreads = t;
         const size_t smem = (size_t)c.r64_smem_slots * 8 + resident64_small_bytes(c.n, c.m, c.r64_check_groups, c.r64_bit_groups);
-        QLB_CUDA(allow_full_dynamic_smem(ctx, kern));
-        long long grid = ctx->sm_count;
-        if (grid > args.n_frames)
-            grid = args.n_frames;
-        const size_t tail = align_up((size_t)(c.slots - c.r64_smem_slots) * 8 + 16, 256);
-        QLB_CUDA(ctx->scratch.reserve((size_t)grid * tail));
-        args.scratch = static_cast<unsigned char *>(ctx->scratch.p);
-        args.scratch_stride = tail;
-#ifdef QLB_DEBUG_LAUNCH
-        std::fprintf(stderr, "[qlb] decode_resident_f64_kernel: %d threads, %u of %d slots in shared memory (%zu B), %zu B tail scratch per CTA, grid=%lld, "
-                             "%d check groups, %d bit groups\n", kThreads, c.r64_smem_slots, c.slots, smem, tail, grid, c.r64_check_groups, c.r64_bit_groups);
-#endif
-        QLB_CUDA(cudaMemsetAsync(ctx->d_counters, 0, sizeof(unsigned long long), ctx->stream));
-        args.queue = ctx->d_counters;
-        args.iter_total = ctx->d_counters + 1;
-        std::snprintf(ctx->last_decoder, sizeof ctx->last_decoder, "resident_f64%s bw=%d threads=%d smem_slots=%u/%d",
+        const size_t tail = align_up((size_t)(c.slots - c.r64_smem_slots) * 8 + 16, 256); // the slots beyond r64_smem_slots
+        char name[sizeof(qlb_ctx::last_decoder)];
+        std::snprintf(name, sizeof name, "resident_f64%s bw=%d threads=%d smem_slots=%u/%d",
                       std::is_same<Math, MathF64Fused>::value ? "fused" : "", kBW, kThreads, c.r64_smem_slots, c.slots);
-        kern<<<(unsigned)grid, kThreads, smem, ctx->stream>>>(args);
-        QLB_CUDA(cudaGetLastError());
-        ++ctx->launches;
-        return QLB_OK;
-    }
-    template <typename Math, bool kReconcile>
-    int launch_resident64_bw(qlb_ctx *ctx, DecodeArgs &args)
-    {
-        switch (args.code.uniform_bit_w)
-        {
-#ifndef QLB_R64_LEAN // kernel-tuning builds (scripts/build_stream_variants.py) compile the bit weight of the benchmark code only
-        case 2: return launch_resident64<Math, kReconcile, 2>(ctx, args);
-        case 4: return launch_resident64<Math, kReconcile, 4>(ctx, args);
-#endif
-        case 3: return launch_resident64<Math, kReconcile, 3>(ctx, args);
-        default: return fail(QLB_ERR_UNSUPPORTED, "fp64 resident kernel: unsupported bit weight");
-        }
+        return launch_persistent(ctx, args, kern, kThreads, smem, 1, tail, name); // one resident CTA per SM
     }
 }
 namespace qlb
 {
-    bool resident_f64_eligible(const qlb_ctx *ctx, const CodeDev &c) { return resident64_eligible_impl(ctx, c) && c.r64_check_group_table; }
-
     // The group tables of the two walks (see qlb_resident_f64.cuh). `bit_slots`: [max_bit_w][n] physical slot of every edge of every bit.
-    // Returns false (and leaves the outputs empty) when the kernel does not take the code on this device.
+    // Returns false (outputs unspecified) when the kernel does not take the code on this device: the kernel's admission test.
     bool resident64_build_tables(const qlb_ctx *ctx, const CodeDev &c, const uint32_t *bit_slots, std::vector<uint32_t> &check_groups,
                                  std::vector<uint16_t> &bit_groups, uint32_t &smem_slots)
     {
-        check_groups.clear();
-        bit_groups.clear();
-        smem_slots = 0;
-        if (!resident64_eligible_impl(ctx, c))
-            return false;
         smem_slots = resident64_smem_slots(ctx, c);
+        if (!(c.slots < 65535 && c.n < 65536 && c.m < 65536 && c.bit_slots16 && c.col_of_slot16 && c.uniform_bit_w >= 2 && c.uniform_bit_w <= 4 &&
+              c.max_check_w <= kResidentMaxCW && c.n % 32 == 0 && smem_slots >= (uint32_t)c.slots / 2))
+            return false;
         std::vector<uint32_t> slow, fast;
         auto push_run = [&](uint32_t lo, uint32_t hi, int w, int tail)
         {
@@ -122,10 +80,7 @@ namespace qlb
         check_groups = slow;
         check_groups.insert(check_groups.end(), fast.begin(), fast.end());
         if ((int)check_groups.size() > check_group_cap(c))
-        {
-            check_groups.clear();
             return false;
-        }
         std::vector<uint16_t> bslow, bfast;
         for (int g = 0; g < c.n / 32; ++g)
         {
@@ -144,10 +99,21 @@ namespace qlb
         return true;
     }
 
-    int launch_resident_f64(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fused)
+    int launch_resident_f64(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        if (fused)
-            return reconcile ? launch_resident64_bw<MathF64Fused, true>(ctx, args) : launch_resident64_bw<MathF64Fused, false>(ctx, args);
-        return reconcile ? launch_resident64_bw<MathF64, true>(ctx, args) : launch_resident64_bw<MathF64, false>(ctx, args);
+        return with_rule<Rule::F64, Rule::F64Fused>(r, [&](auto rule, auto reconcile) -> int
+        {
+            typedef MathOf<decltype(rule)::value> Math;
+            constexpr bool kReconcile = decltype(reconcile)::value;
+            switch (args.code.uniform_bit_w)
+            {
+#ifndef QLB_R64_LEAN // kernel-tuning builds (scripts/build_stream_variants.py) compile the bit weight of the benchmark code only
+            case 2: return launch_resident64<Math, kReconcile, 2>(ctx, args, r.block_threads);
+            case 4: return launch_resident64<Math, kReconcile, 4>(ctx, args, r.block_threads);
+#endif
+            case 3: return launch_resident64<Math, kReconcile, 3>(ctx, args, r.block_threads);
+            default: return fail(QLB_ERR_UNSUPPORTED, "fp64 resident kernel: unsupported bit weight");
+            }
+        });
     }
 }

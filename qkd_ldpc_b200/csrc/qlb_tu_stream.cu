@@ -1,5 +1,4 @@
 #include "qlb_internal.hpp"
-#include <algorithm>
 using namespace qlb;
 #include "qlb_stream_split.cuh"
 
@@ -8,7 +7,7 @@ namespace
     // The streaming decoder (qlb_stream_split.cuh): one kernel per pass over all groups, in waves when device memory cannot
     // hold the message arrays of every group at once. Nothing here waits for the device.
     template <typename P, bool kReconcile, int kBW, int VEC>
-    int launch_stream_split(qlb_ctx *ctx, DecodeArgs &args, size_t budget)
+    int launch_stream_split(qlb_ctx *ctx, DecodeArgs &args, const Route &r, size_t budget)
     {
         typedef typename P::real Real;
         const long long G = 32 * VEC, groups = (args.n_frames + G - 1) / G;
@@ -20,8 +19,8 @@ namespace
             return fail(QLB_ERR_UNSUPPORTED, "streaming decoder: more than 2^32 message values per frame group");
         const size_t per_bundle = split_bundle_bytes(args.code.n, args.code.m, args.code.slots, VEC, B, (int)sizeof(Real));
         long long fit_bundles = (long long)(budget / per_bundle);
-        if (args.stream_max_bundles > 0) // qlb_decode_params.stream_max_bundles: waves without filling the device memory
-            fit_bundles = std::min<long long>(fit_bundles, args.stream_max_bundles);
+        if (r.stream_max_bundles > 0) // qlb_decode_params.stream_max_bundles: waves without filling the device memory
+            fit_bundles = std::min<long long>(fit_bundles, r.stream_max_bundles);
         if (fit_bundles < 1)
             return fail(QLB_ERR_UNSUPPORTED, "streaming decoder: device memory cannot hold the messages of one bundle of frame groups");
         const long long bundles = (groups + B - 1) / B;
@@ -53,8 +52,6 @@ namespace
         st.fmap_new = st.src_of + (size_t)per_wave * G;
         if (args.syndrome_out)
             QLB_CUDA(cudaMemsetAsync(args.syndrome_out, 0, (size_t)args.n_frames * args.code.words_m * 4, ctx->stream));
-        args.queue = ctx->d_counters;
-        args.iter_total = ctx->d_counters + 1;
 
         auto k_setup = stream_setup_kernel<Real, kReconcile, VEC>;
         auto k_init = stream_init_kernel<P, kReconcile, kBW, VEC>;
@@ -67,7 +64,7 @@ namespace
         auto k_mvbits = stream_repack_bits_kernel<Real, VEC>;
         auto k_commit = stream_repack_commit_kernel<VEC>;
         // rounds after which a repack is attempted (decided on the device: live columns <= half of the streamed ones)
-        const bool repack_on = !args.stream_no_repack && per_wave <= kMaxRepackGroups && per_wave >= 2;
+        const bool repack_on = !r.stream_no_repack && per_wave <= kMaxRepackGroups && per_wave >= 2;
         // attempts every 2 / 3 / 4 rounds measured 0.681 / 0.680 / 0.681 at the waterfall, but every second round costs the
         // early-converging QBERs 10 %; a declined attempt costs ~15 us
         auto repack_round = [](int it) { return it >= 4 && it % 4 == 2; };
@@ -117,28 +114,18 @@ namespace
     }
 
     template <typename P, bool kReconcile, int kBW>
-    int launch_stream_vec(qlb_ctx *ctx, DecodeArgs &args)
+    int launch_stream_vec(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
         size_t free_b = 0, total_b = 0;
         QLB_CUDA(cudaMemGetInfo(&free_b, &total_b));
         const size_t budget = (free_b + ctx->scratch.cap) / 20 * 17;
         // groups of 128 (fp32) / 64 (fp64) frames: 128-bit accesses; a batch of <= 32 frames takes 32-frame groups
-        return args.n_frames > 32 ? launch_stream_split<P, kReconcile, kBW, P::kVecWide>(ctx, args, budget) : launch_stream_split<P, kReconcile, kBW, 1>(ctx, args, budget);
+        return args.n_frames > 32 ? launch_stream_split<P, kReconcile, kBW, P::kVecWide>(ctx, args, r, budget) : launch_stream_split<P, kReconcile, kBW, 1>(ctx, args, r, budget);
     }
 
-    template <typename P, bool kReconcile>
-    int launch_stream_bw(qlb_ctx *ctx, DecodeArgs &args)
-    {
-        switch (args.code.uniform_bit_w)
-        {
-#ifndef QLB_STREAM_LEAN // kernel-tuning builds (scripts/build_stream_variants.py) compile the bit weight of the benchmark codes only
-        case 2: return launch_stream_vec<P, kReconcile, 2>(ctx, args);
-        case 4: return launch_stream_vec<P, kReconcile, 4>(ctx, args);
-#endif
-        case 3: return launch_stream_vec<P, kReconcile, 3>(ctx, args);
-        default: return launch_stream_vec<P, kReconcile, 0>(ctx, args); // irregular or heavier bits: the any-weight bit pass
-        }
-    }
+    // The streaming kernels' form of each rule (qlb_stream_common.cuh).
+    template <Rule kRule>
+    using StreamOf = std::tuple_element_t<(int)kRule, std::tuple<StreamF64<MathF64>, StreamF64<MathF64Fused>, StreamF32<RuleF32Accurate>, StreamF32<RuleF32Fast>>>;
 }
 namespace qlb
 {
@@ -148,16 +135,21 @@ namespace qlb
     {
         return c.max_bit_w >= 1 && c.max_check_w <= kResidentMaxCW && c.m <= c.n && c.col_of_slot32 != nullptr;
     }
-    int launch_stream_f32(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fast)
+    int launch_stream(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        if (fast)
-            return reconcile ? launch_stream_bw<StreamF32<RuleF32Fast>, true>(ctx, args) : launch_stream_bw<StreamF32<RuleF32Fast>, false>(ctx, args);
-        return reconcile ? launch_stream_bw<StreamF32<RuleF32Accurate>, true>(ctx, args) : launch_stream_bw<StreamF32<RuleF32Accurate>, false>(ctx, args);
-    }
-    int launch_stream_f64(qlb_ctx *ctx, DecodeArgs &args, bool reconcile, bool fused)
-    {
-        if (fused)
-            return reconcile ? launch_stream_bw<StreamF64<MathF64Fused>, true>(ctx, args) : launch_stream_bw<StreamF64<MathF64Fused>, false>(ctx, args);
-        return reconcile ? launch_stream_bw<StreamF64<MathF64>, true>(ctx, args) : launch_stream_bw<StreamF64<MathF64>, false>(ctx, args);
+        return with_rule<Rule::F64, Rule::F64Fused, Rule::F32, Rule::F32Fast>(r, [&](auto rule, auto reconcile) -> int
+        {
+            typedef StreamOf<decltype(rule)::value> P;
+            constexpr bool kReconcile = decltype(reconcile)::value;
+            switch (args.code.uniform_bit_w)
+            {
+#ifndef QLB_STREAM_LEAN // kernel-tuning builds (scripts/build_stream_variants.py) compile the bit weight of the benchmark codes only
+            case 2: return launch_stream_vec<P, kReconcile, 2>(ctx, args, r);
+            case 4: return launch_stream_vec<P, kReconcile, 4>(ctx, args, r);
+#endif
+            case 3: return launch_stream_vec<P, kReconcile, 3>(ctx, args, r);
+            default: return launch_stream_vec<P, kReconcile, 0>(ctx, args, r); // irregular or heavier bits: the any-weight bit pass
+            }
+        });
     }
 }

@@ -7,13 +7,8 @@
 set -e
 cd "$(dirname "$0")/.."
 if [ "$1" = build ]; then
-  for tu in qlb_api qlb_tu_resident_f32 qlb_tu_resident_f64 qlb_tu_stream; do
-    nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -ccbin /usr/bin/g++ -Xcompiler -fPIC -DQLB_BOUNDS_CHECK -DQLB_STREAM_LEAN \
-      -c -o qkd_ldpc_b200/lib/variants/bounds_$tu.o qkd_ldpc_b200/csrc/$tu.cu &
-  done
-  wait
-  nvcc -gencode arch=compute_100a,code=sm_100a -shared -ccbin /usr/bin/g++ -o qkd_ldpc_b200/lib/variants/libbounds.so qkd_ldpc_b200/lib/variants/bounds_*.o -ldl
-  rm -f qkd_ldpc_b200/lib/variants/bounds_*.o
+  python -c 'from qkd_ldpc_b200 import build as b
+b.build_library(force=True, verbose_ptxas=False, out=b.LIB_DIR / "variants" / "libbounds.so", extra_flags=["-DQLB_BOUNDS_CHECK", "-DQLB_STREAM_LEAN"])'
   ls -la qkd_ldpc_b200/lib/variants/libbounds.so
 else
   export QLB_LIBRARY=$PWD/qkd_ldpc_b200/lib/variants/libbounds.so

@@ -4,12 +4,7 @@
 set -e
 cd "$(dirname "$0")/.."
 TAG=$1; FLAGS=$2
-mkdir -p qkd_ldpc_b200/lib/variants
-for tu in qlb_api qlb_tu_resident_f32 qlb_tu_resident_f64 qlb_tu_stream; do
-  nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -ccbin /usr/bin/g++ -Xcompiler -fPIC $FLAGS \
-    -c -o qkd_ldpc_b200/lib/variants/${TAG}_$tu.o qkd_ldpc_b200/csrc/$tu.cu &
-done
-wait
-nvcc -gencode arch=compute_100a,code=sm_100a -shared -ccbin /usr/bin/g++ -o qkd_ldpc_b200/lib/variants/lib$TAG.so qkd_ldpc_b200/lib/variants/${TAG}_*.o -ldl
-rm -f qkd_ldpc_b200/lib/variants/${TAG}_*.o
+python -c 'import sys
+from qkd_ldpc_b200 import build as b
+b.build_library(force=True, verbose_ptxas=False, out=b.LIB_DIR / "variants" / f"lib{sys.argv[1]}.so", extra_flags=sys.argv[2].split())' "$TAG" "$FLAGS"
 ls -la qkd_ldpc_b200/lib/variants/lib$TAG.so

@@ -447,3 +447,24 @@ def test_resident_f64_block_threads(ctx, oracle):
                                            want_decoded=True, want_syndrome=True)
                 assert f"threads={t} " in ctx.last_decoder and ctx.last_decoder.startswith("resident_f64"), (t, ctx.last_decoder)
                 assert all((x == y).all() for x, y in zip(ref, got)), (key, fused, t)
+
+
+# ---- f. the test hook -------------------------------------------------------------------------------------------------------------
+def test_test_hook_above_3_is_rejected(ctx, oracle):
+    """qlb_decode_params.flags bits 8..11 hold 1 + the test hook: 0 ... 2 force a generic kernel storage tier, 3 the streaming
+    decoder. A larger hook is invalid input (QLB_ERR_INVALID) in every decode entry, in both precisions."""
+    mat, g, code = code_of("perm3_n1024")
+    seeds = oracle.trial_seeds(11, 4)
+    a, b, ex = ctx.generate(mat.n, seeds, 0.05)
+    llr = np.full((4, mat.n), 2.0)
+    syn = np.zeros((4, mat.m), np.int32)
+    for precision in (64, 32):
+        ctx.reconcile_packed(code, capi.make_params(precision, 10, 100.0, True, tier=3), a, b, np.full(4, ex))
+        assert ctx.last_decoder.startswith(f"stream_f{precision}"), ctx.last_decoder
+        for hook in (4, 14):
+            p = capi.make_params(precision, 10, 100.0, True, tier=hook)
+            for call in (lambda: ctx.reconcile_packed(code, p, a, b, np.full(4, ex)), lambda: ctx.sum_product(code, p, llr, syn),
+                         lambda: ctx.run_trials(code, p, seeds, 0.05)):
+                with pytest.raises(capi.QlbError) as ei:
+                    call()
+                assert ei.value.code == 1 and "test hook" in ei.value.message, (precision, hook, str(ei.value))
