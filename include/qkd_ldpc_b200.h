@@ -34,7 +34,9 @@
 extern "C" {
 #endif
 
-#define QLB_VERSION 200 /* 0.2.0: qlb_decode_params grew execution knobs (was 24 bytes, now 40) */
+/* 0.2.0: qlb_decode_params grew execution knobs (was 24 bytes, now 40);
+ * 0.3.0: QLB_FLAG_F32_MIN_SUM, and qlb_decode_params.reserved became min_sum_scale (same size and offsets) */
+#define QLB_VERSION 300
 
 /* status codes (0 = ok); qlb_last_error() gives the message of the calling thread's last failure */
 enum {
@@ -60,6 +62,22 @@ enum {
      * by the SM-resident fp64 kernel and by the generic kernel (checks wider than its unrolled shapes keep the literal order).
      * Per-frame outcomes validated against the reference in profiles/parity_r01.md and on the exhaustive small-code fixtures. */
     QLB_FLAG_F64_FUSED_RATIO = 2,
+    /* fp32 only, not with QLB_FLAG_F32_FAST_MATH: the normalized min-sum check rule with scale alpha =
+     * qlb_decode_params.min_sum_scale in (0, 1]. No transcendental function is involved, so every decoder that runs it gives
+     * the same result on every frame (iterations, flags, decoded bits), equal to a plain-C restatement on the CPU. The rule:
+     *   - messages are fp32 in natural-log units: the prior is +-(float)log_prior (reconcile) or (float)llr (sum-product;
+     *     a NaN LLR enters as the fp32 NaN 0x7FFFFFFF);
+     *   - bit 0 of a bit->check message word carries a bit: Alice's bit (reconcile) or 0 (sum-product) in the first messages,
+     *     (bits(prior) & ~1) | a; after each bit pass the sender's hard decision z, (bits(extrinsic) & ~1) | z;
+     *   - check j of weight w, syndrome bit s, incoming words u_0 ... u_{w-1}: X = (s << 31) ^ u_0 ^ ... ^ u_{w-1}. Edge k
+     *     gets sign bit 31 of X ^ u_k and magnitude fminf(alpha * mu_k, cap), one round-to-nearest fp32 multiply, where
+     *     mu_k = the minimum over i != k of (u_i & 0x7FFFFFFF) compared as unsigned integers (the float order, NaN above
+     *     +inf; the empty minimum of a weight-1 check is +inf) and cap = (float)threshold, or +inf when the clamp is off.
+     *     fminf(NaN, cap) = cap, so a check sends no NaN;
+     *   - bit pass: total = prior + c_0 + c_1 + ... in the reference's arrival order (fp32 adds, no FMA), z = total <= 0,
+     *     extrinsic fminf(fmaxf(total - c_k, -cap), cap) -- also with the clamp off, so a NaN total (inf - inf) sends -cap;
+     *   - iterations, flags, decoded key and Alice's syndrome as for every other rule. */
+    QLB_FLAG_F32_MIN_SUM = 4,
     /* test hook, bits 8..11 = 1 + hook (0: no hook). Hooks 0 / 1 / 2 run the generic kernel in that storage tier (0 shared
      * memory, 1 L2 scratch for messages, 2 all global) instead of the fastest eligible decoder; a tier faster than the fastest
      * the code fits in is ignored. Hook 3 runs the streaming decoder, or fails with QLB_ERR_UNSUPPORTED when it does not take
@@ -83,7 +101,7 @@ typedef struct qlb_decode_params {
     int32_t stream_max_bundles; /* streaming decoder: at most this many 4-group bundles per wave (default: what device memory holds) */
     int32_t stream_no_repack;   /* streaming decoder: 1 = no on-device compaction of the live frames                  */
     int32_t block_threads;      /* SM-resident decoders: threads per CTA (multiple of 32; ignored when inadmissible)   */
-    int32_t reserved;           /* must be 0                                                                           */
+    float min_sum_scale;        /* QLB_FLAG_F32_MIN_SUM: the scale alpha in (0, 1]; must be 0 without the flag         */
 } qlb_decode_params;
 
 /* Per-frame result of a decode; mirrors SP_result / LDPC_result (src/qkd_ldpc_algorithm.hpp:14-24). */
@@ -136,10 +154,10 @@ int qlb_ctx_sm_count(const qlb_ctx *ctx);
 /* The context's CUDA stream (a cudaStream_t) for callers that time or order work with their own events. */
 void *qlb_ctx_stream(const qlb_ctx *ctx);
 /* Which decoder the context's last decode launched, written by the launcher itself (empty before the first decode):
- *   "generic f64|f64fused|f32|f32fast tier=T shape=S threads=K"       the generic kernel (storage tier, unrolled check shape)
+ *   "generic f64|f64fused|f32|f32fast|f32minsum tier=T shape=S threads=K"  the generic kernel (storage tier, unrolled check shape)
  *   "resident_f64[fused] bw=B threads=K smem_slots=X/S"             the SM-resident fp64 kernel (X of S message slots in shared memory)
- *   "resident_f32[fast] bw=B threads=K"                             the SM-resident fp32 kernel
- *   "stream_f32|f64 vec=V bw=B|any bundle=B waves=W repack=0|1"     the streaming decoder
+ *   "resident_f32[fast|minsum] bw=B threads=K"                      the SM-resident fp32 kernel
+ *   "stream_f32|f64 vec=V bw=B|any bundle=B waves=W repack=0|1"     the streaming decoder (the string names no fp32 rule)
  * The string is owned by the context and valid until its next decode. */
 const char *qlb_ctx_last_decoder(const qlb_ctx *ctx);
 int qlb_ctx_synchronize(qlb_ctx *ctx);

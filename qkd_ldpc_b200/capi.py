@@ -17,6 +17,7 @@ PRECISION_F64 = 64
 PRECISION_F32 = 32
 FLAG_F32_FAST_MATH = 1
 FLAG_F64_FUSED_RATIO = 2
+FLAG_F32_MIN_SUM = 4
 RES_SYNDROMES_MATCH = 1
 RES_KEYS_MATCH = 2
 
@@ -50,7 +51,7 @@ class DecodeParams(C.Structure):
         ("stream_max_bundles", C.c_int32),
         ("stream_no_repack", C.c_int32),
         ("block_threads", C.c_int32),
-        ("reserved", C.c_int32),
+        ("min_sum_scale", C.c_float),
     ]
 
 
@@ -125,15 +126,20 @@ def _ptr(a):
 
 
 def make_params(precision=64, max_iterations=100, threshold=100.0, enable_threshold=True, fast_math=False, tier=None,
-                stream_max_bundles=0, stream_no_repack=False, block_threads=0):
+                stream_max_bundles=0, stream_no_repack=False, block_threads=0, min_sum_scale=None):
+    """min_sum_scale: the scale alpha in (0, 1] of the fp32 normalized min-sum check rule (QLB_FLAG_F32_MIN_SUM); None: the
+    precision's sum-product rule."""
     if fast_math:  # the cheaper check rule of either precision
         flags = FLAG_F32_FAST_MATH if int(precision) == 32 else FLAG_F64_FUSED_RATIO
     else:
         flags = 0
+    if min_sum_scale is not None:
+        flags |= FLAG_F32_MIN_SUM
     if tier is not None:
         flags |= (int(tier) + 1) << 8  # QLB_FLAG_TEST_TIER_SHIFT hook: 0 ... 2 a generic kernel storage tier, 3 the streaming decoder
     return DecodeParams(int(precision), int(max_iterations), int(bool(enable_threshold)), flags, float(threshold),
-                        int(stream_max_bundles), int(bool(stream_no_repack)), int(block_threads), 0)
+                        int(stream_max_bundles), int(bool(stream_no_repack)), int(block_threads),
+                        0.0 if min_sum_scale is None else float(min_sum_scale))
 
 
 def pack_bits(bits, n=None) -> np.ndarray:

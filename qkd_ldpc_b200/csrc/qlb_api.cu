@@ -178,8 +178,19 @@ namespace
             return fail(QLB_ERR_INVALID, "QLB_FLAG_F32_FAST_MATH requires fp32 precision");
         if ((p->flags & QLB_FLAG_F64_FUSED_RATIO) && p->precision != QLB_PRECISION_F64)
             return fail(QLB_ERR_INVALID, "QLB_FLAG_F64_FUSED_RATIO requires fp64 precision");
-        if (p->stream_max_bundles < 0 || p->block_threads < 0 || p->reserved != 0)
-            return fail(QLB_ERR_INVALID, "qlb_decode_params: negative execution knob or non-zero reserved field");
+        if (p->stream_max_bundles < 0 || p->block_threads < 0)
+            return fail(QLB_ERR_INVALID, "qlb_decode_params: negative execution knob");
+        if (p->flags & QLB_FLAG_F32_MIN_SUM)
+        {
+            if (p->precision != QLB_PRECISION_F32)
+                return fail(QLB_ERR_INVALID, "QLB_FLAG_F32_MIN_SUM requires fp32 precision");
+            if (p->flags & QLB_FLAG_F32_FAST_MATH)
+                return fail(QLB_ERR_INVALID, "QLB_FLAG_F32_MIN_SUM and QLB_FLAG_F32_FAST_MATH exclude each other");
+            if (!(p->min_sum_scale > 0.f && p->min_sum_scale <= 1.f))
+                return fail(QLB_ERR_INVALID, "qlb_decode_params.min_sum_scale must be in (0, 1] with QLB_FLAG_F32_MIN_SUM");
+        }
+        else if (p->min_sum_scale != 0.f) // also a NaN
+            return fail(QLB_ERR_INVALID, "qlb_decode_params.min_sum_scale must be 0 without QLB_FLAG_F32_MIN_SUM");
         if (((p->flags >> QLB_FLAG_TEST_TIER_SHIFT) & 0xF) > 4)
             return fail(QLB_ERR_INVALID, "qlb_decode_params.flags: the test hook (bits 8..11) must be 0 (none) or 1 + hook, hook 0 ... 3");
         return QLB_OK;

@@ -99,7 +99,8 @@ namespace qlb
         return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - (int)fa.sharedSizeBytes);
     }
 
-    enum class Rule { F64, F64Fused, F32, F32Fast }; // the precision and its cheaper check rule (QLB_FLAG_F32_FAST_MATH / F64_FUSED_RATIO)
+    // the precision and its cheaper check rule (QLB_FLAG_F32_FAST_MATH / F64_FUSED_RATIO), or fp32 min-sum (QLB_FLAG_F32_MIN_SUM)
+    enum class Rule { F64, F64Fused, F32, F32Fast, F32MinSum };
     enum class Family { ResidentF32, ResidentF64, Stream, Generic };
     struct Route // the decoder that takes a batch, and how it runs
     {
@@ -122,7 +123,7 @@ namespace qlb
     int launch_generic(qlb_ctx *ctx, DecodeArgs &args, const Route &r);
 
     // The node arithmetic (qlb_kernels.cuh) of each rule in the generic kernel and the fp64 decoders.
-    template <Rule kRule> using MathOf = std::tuple_element_t<(int)kRule, std::tuple<MathF64, MathF64Fused, MathF32, MathF32Fast>>;
+    template <Rule kRule> using MathOf = std::tuple_element_t<(int)kRule, std::tuple<MathF64, MathF64Fused, MathF32, MathF32Fast, MathF32MinSum>>;
 
     // Calls f(rule, reconcile) with the route's rule and mode as std::integral_constant<Rule, ...> and std::bool_constant: template
     // arguments for a launcher. Only the listed rules, those the family implements (route_decode picks no other), are instantiated.
@@ -172,6 +173,8 @@ namespace qlb
         Rule rule = fp32 ? Rule::F32 : Rule::F64;
         if (p.flags & (fp32 ? QLB_FLAG_F32_FAST_MATH : QLB_FLAG_F64_FUSED_RATIO)) // the precision's cheaper check rule
             rule = fp32 ? Rule::F32Fast : Rule::F64Fused;
+        if (p.flags & QLB_FLAG_F32_MIN_SUM) // fp32 only, never with the fast rule (check_params)
+            rule = Rule::F32MinSum;
         out = Route{Family::Generic, rule, reconcile, kTierGlobal, p.stream_max_bundles, p.stream_no_repack, p.block_threads};
         if (hook < 0 && (fp32 ? resident_f32_eligible(ctx, c) : c.r64_check_group_table != nullptr))
             out.family = fp32 ? Family::ResidentF32 : Family::ResidentF64;
@@ -198,6 +201,7 @@ namespace qlb
         args.enable_thr = p.enable_threshold;
         args.thr = p.threshold;
         args.cap_f32 = p.enable_threshold ? (float)p.threshold : INFINITY;
+        args.ms_scale = p.min_sum_scale;
         switch (r.family)
         {
         case Family::ResidentF32: return launch_resident_f32(ctx, args, r);

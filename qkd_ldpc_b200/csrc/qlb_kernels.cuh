@@ -82,6 +82,7 @@ namespace qlb
         int32_t max_it;
         int32_t enable_thr;
         float cap_f32; // (float)thr, or +inf when the clamp is disabled
+        float ms_scale; // the min-sum scale alpha (QLB_FLAG_F32_MIN_SUM; 0 for the other rules), in the hole before thr
         double thr;
         // reconcile mode
         const uint32_t *alice;    // [F][words_n]
@@ -378,6 +379,56 @@ namespace qlb
         }
     };
 
+    // fp32 normalized min-sum (QLB_FLAG_F32_MIN_SUM), defined to the bit in include/qkd_ldpc_b200.h. Messages are raw words: bit 0
+    // of a bit->check word carries a bit (Alice's bit, then the sender's hard decision), and the check rule reads it as part of
+    // the magnitude. The pieces below are shared by every decoder that runs the rule.
+    struct MathF32MinSum
+    {
+        typedef float real;
+        // one incoming word: x ^= u; m1 <= m2 = the two smallest magnitude words so far as unsigned integers. Both start at +inf
+        // (0x7F800000) instead of above every NaN, which changes no output: a minimum of +inf or NaN gives fminf(inf or NaN, cap) = cap.
+        static __device__ __forceinline__ void take(uint32_t u, uint32_t &x, uint32_t &m1, uint32_t &m2)
+        {
+            const uint32_t a = u & 0x7FFFFFFFu;
+            x ^= u;
+            m2 = min(m2, max(m1, a));
+            m1 = min(m1, a);
+        }
+        // The word sent on edges whose own magnitude is not the minimum (from m = m1) and on the edge that holds it (m = m2),
+        // with the sign bit of x = (syndrome bit << 31) ^ every incoming word; out() then flips it by the edge's own sign.
+        static __device__ __forceinline__ uint32_t word(uint32_t m, uint32_t x, float cap, float scale)
+        {
+            return __float_as_uint(fminf(__fmul_rn(scale, __uint_as_float(m)), cap)) | (x & 0x80000000u);
+        }
+        // the outgoing word of the edge whose incoming word is u: one compare, one select, one LOP3
+        static __device__ __forceinline__ float out(uint32_t u, uint32_t m1, uint32_t w1, uint32_t w2)
+        {
+            return __uint_as_float(((u & 0x7FFFFFFFu) == m1 ? w2 : w1) ^ (u & 0x80000000u));
+        }
+        // the bit->check word: the extrinsic value clamped (cap = +inf when the clamp is off: a NaN still becomes -cap), bit 0 = z
+        static __device__ __forceinline__ float b2c(float v, float cap, bool z)
+        {
+            v = fminf(fmaxf(v, -cap), cap);
+            return __uint_as_float((__float_as_uint(v) & ~1u) | (uint32_t)z);
+        }
+        // the first message of a bit: bit 0 = Alice's bit (reconcile mode) or 0
+        static __device__ __forceinline__ float first(float prior, uint32_t abit) { return __uint_as_float((__float_as_uint(prior) & ~1u) | abit); }
+        template <int W>
+        static __device__ __forceinline__ void check(float (&v)[W], int w, bool s, float cap, float scale)
+        {
+            uint32_t x = s ? 0x80000000u : 0u, m1 = 0x7F800000u, m2 = 0x7F800000u;
+#pragma unroll
+            for (int k = 0; k < W; ++k)
+                if (k < w)
+                    take(__float_as_uint(v[k]), x, m1, m2);
+            const uint32_t w1 = word(m1, x, cap, scale), w2 = word(m2, x, cap, scale);
+#pragma unroll
+            for (int k = 0; k < W; ++k)
+                if (k < w)
+                    v[k] = out(__float_as_uint(v[k]), m1, w1, w2);
+        }
+    };
+
     // two-pass helpers for the generic (any weight) path of the fp32 rules: divide form with explicit zero handling,
     // equivalent to the leave-one-out product
     template <typename Math>
@@ -497,6 +548,7 @@ namespace qlb
         constexpr uint32_t kNone = IdxTraits<IdxT>::kNone;
         constexpr int W = kShapeW == 0 ? 1 : kShapeW;
         constexpr int WV = 4;
+        constexpr bool kMinSum = std::is_same<Math, MathF32MinSum>::value; // raw message words, bit 0 carries a bit (see MathF32MinSum)
 
         extern __shared__ __align__(16) unsigned char smem[];
         const CodeDev &code = args.code;
@@ -577,8 +629,12 @@ namespace qlb
                     abit = (unsigned char)((s_alice[i >> 5] >> (i & 31)) & 1u);
                     prior = bb ? -lp : lp; // :401-405
                 }
+                else if constexpr (kMinSum)
+                    prior = __fmul_rn(1.f, (float)llr_f[i]); // the prior every fp32 kernel forms
                 else
                     prior = (Real)llr_f[i];
+                if constexpr (kMinSum)
+                    prior = MathF32MinSum::first(prior, abit);
                 for (int a = 0; a < max_bw; ++a)
                 {
                     const uint32_t s = bit_slots[(size_t)a * n + i];
@@ -642,11 +698,25 @@ namespace qlb
                                 v[k] = msg[code.base[k] + p];
                                 w = k + 1;
                             }
-                        Math::template check<W>(v, w, s, en, thr);
+                        if constexpr (kMinSum)
+                            Math::template check<W>(v, w, s, args.cap_f32, args.ms_scale);
+                        else
+                            Math::template check<W>(v, w, s, en, thr);
 #pragma unroll
                         for (int k = 0; k < W; ++k)
                             if (k < w)
                                 msg[code.base[k] + p] = v[k];
+                    }
+                    else if constexpr (kMinSum)
+                    {
+                        uint32_t x = s ? 0x80000000u : 0u, m1 = 0x7F800000u, m2 = 0x7F800000u;
+                        for (int k = 0; k < max_cw; ++k)
+                            if ((uint32_t)p < code.cnt[k])
+                                Math::take(__float_as_uint(msg[code.base[k] + p]), x, m1, m2);
+                        const uint32_t w1 = Math::word(m1, x, args.cap_f32, args.ms_scale), w2 = Math::word(m2, x, args.cap_f32, args.ms_scale);
+                        for (int k = 0; k < max_cw; ++k)
+                            if ((uint32_t)p < code.cnt[k])
+                                msg[code.base[k] + p] = Math::out(__float_as_uint(msg[code.base[k] + p]), m1, w1, w2);
                     }
                     else
                     {
@@ -691,6 +761,8 @@ namespace qlb
                         Real prior;
                         if (kReconcile)
                             prior = ((s_bob[i >> 5] >> (i & 31)) & 1u) ? -lp : lp;
+                        else if constexpr (kMinSum)
+                            prior = __fmul_rn(1.f, (float)llr_f[i]);
                         else
                             prior = (Real)llr_f[i];
                         Real total = prior;
@@ -715,7 +787,10 @@ namespace qlb
                             for (int a = 0; a < WV; ++a)
                                 if (sl[a] != kNone)
                                 {
-                                    msg[sl[a]] = clamp_msg(total - c[a], thr, en);
+                                    if constexpr (kMinSum)
+                                        msg[sl[a]] = MathF32MinSum::b2c(total - c[a], args.cap_f32, z);
+                                    else
+                                        msg[sl[a]] = clamp_msg(total - c[a], thr, en);
                                     zedge[sl[a]] = (unsigned char)z;
                                 }
                         }
@@ -733,7 +808,10 @@ namespace qlb
                                 const uint32_t s = bit_slots[(size_t)a * n + i];
                                 if (s != kNone)
                                 {
-                                    msg[s] = clamp_msg(total - msg[s], thr, en);
+                                    if constexpr (kMinSum)
+                                        msg[s] = MathF32MinSum::b2c(total - msg[s], args.cap_f32, z);
+                                    else
+                                        msg[s] = clamp_msg(total - msg[s], thr, en);
                                     zedge[s] = (unsigned char)z;
                                 }
                             }

@@ -85,8 +85,12 @@ namespace qlb
     // ---- check rules for a check of weight exactly W -------------------------------------------------------------------
     // v[] holds the raw incoming messages and receives the outgoing ones. xr = XOR of the raw message words, with the
     // check's syndrome bit folded into bit 31 (sign of the seeded product, src/qkd_ldpc_algorithm.cpp:231).
+    // Arg: what apply() takes besides the messages, formed once per launch by check_arg(cap, DecodeArgs::ms_scale) -- the clamp
+    // in message units for the sum-product rules, the clamp and the scale for min-sum.
     struct RuleF32Fast
     {
+        typedef float Arg;
+        static __device__ __forceinline__ Arg check_arg(float cap, float) { return cap; }
         // Messages are kept in base-2 units (LLR / ln 2): with e = 2^-|m|, tanh(|m| ln2 / 2) = (1-e)/(1+e). For the whole
         // check A = prod(1-e_j), B = prod(1+e_j), S = B + A, D = B - A; the leave-one-out ratio of edge k follows without
         // a division or prefix/suffix products:
@@ -129,6 +133,8 @@ namespace qlb
 
     struct RuleF32Accurate
     {
+        typedef float Arg;
+        static __device__ __forceinline__ Arg check_arg(float cap, float) { return cap; }
         static constexpr float kUnit = 1.f; // natural-log units
         static constexpr bool kParityFirst = true;
         // libdevice tanhf / atanhf, leave-one-out product by prefix * suffix
@@ -160,6 +166,36 @@ namespace qlb
         }
     };
 
+    // Normalized min-sum (QLB_FLAG_F32_MIN_SUM; the rule is defined to the bit in include/qkd_ldpc_b200.h, its pieces are
+    // MathF32MinSum's). Per edge: a mask, two integer min/max, one compare, one select, one LOP3 for the sign; per check: two
+    // multiplies and two fminf. Every operation is exact or one IEEE rounding, so the result equals the CPU restatement's
+    // (tests/min_sum_restatement.c) on every frame.
+    struct RuleF32MinSum
+    {
+        struct Arg
+        {
+            float cap, scale;
+        };
+        static __device__ __forceinline__ Arg check_arg(float cap, float scale) { return Arg{cap, scale}; }
+        // natural-log units: the clamp and the priors mean what they mean for the accurate rule, and the bit pass always clamps
+        static constexpr float kUnit = 1.f;
+        // No parity-first look: it pays for rules whose check pass is expensive, and this check pass is cheaper than the fast
+        // rule's, for which the look already measured no gain (RuleF32Fast) -- its extra live state would cost the hot loops more.
+        static constexpr bool kParityFirst = false;
+        template <int W>
+        static __device__ __forceinline__ void apply(float (&v)[W], uint32_t xr, Arg a)
+        {
+            uint32_t x = 0, m1 = 0x7F800000u, m2 = 0x7F800000u; // x: unused, the caller's xr already holds the XOR
+#pragma unroll
+            for (int k = 0; k < W; ++k)
+                MathF32MinSum::take(__float_as_uint(v[k]), x, m1, m2);
+            const uint32_t w1 = MathF32MinSum::word(m1, xr, a.cap, a.scale), w2 = MathF32MinSum::word(m2, xr, a.cap, a.scale);
+#pragma unroll
+            for (int k = 0; k < W; ++k)
+                v[k] = MathF32MinSum::out(__float_as_uint(v[k]), m1, w1, w2);
+        }
+    };
+
     // Where the byte offset of edge position k's slot row comes from: the kernel parameters (constant bank, a free operand
     // for compile-time k) on the hot path, a shared-memory copy for the out-of-line wide weights.
     struct BaseFromParams
@@ -180,7 +216,7 @@ namespace qlb
     // Returns the OR over the thread's checks of (parity of the riding hard decisions) ^ (syndrome bit), in bit 0.
     template <typename Rule, int W, typename Base>
     __device__ __forceinline__ uint32_t check_segment(const int kThreads, unsigned char *__restrict__ msg_bytes, const Base base4, uint32_t lo, uint32_t hi,
-                                                      uint32_t my_syn, int &rbit, float cap)
+                                                      uint32_t my_syn, int &rbit, typename Rule::Arg cap)
     {
         uint32_t bad = 0;
 #pragma unroll 1
@@ -209,7 +245,7 @@ namespace qlb
     // weights 9..16 are kept out of line: their register appetite must not leak into the hot (narrow) instantiations
     template <typename Rule, int W>
     __device__ __noinline__ uint32_t check_segment_wide(const int kThreads, unsigned char *msg_bytes, const uint32_t *s_base4, uint32_t lo, uint32_t hi,
-                                                        uint32_t my_syn, int rbit, float cap)
+                                                        uint32_t my_syn, int rbit, typename Rule::Arg cap)
     {
         const uint32_t bad = check_segment<Rule, W>(kThreads, msg_bytes, BaseFromSmem{s_base4}, lo, hi, my_syn, rbit, cap);
         return (bad & 1u) | ((uint32_t)rbit << 1); // bit 0: parity failure, bits 1..: advanced round counter
@@ -370,6 +406,7 @@ namespace qlb
         // messages at a threshold >= 25 base-2 units cannot change any later value, so that clamp is skipped.
         const bool clamp_b2c = !(Rule::kUnit != 1.f && cap >= 25.f);
         const int nseg = s_nseg;
+        const typename Rule::Arg rule_arg = Rule::check_arg(cap, args.ms_scale);
 
         for (;;)
         {
@@ -484,8 +521,8 @@ namespace qlb
                         const uint32_t lo = s_seg_lo[sg], hi = s_seg_hi[sg];
                         switch (s_seg_w[sg])
                         {
-#define QLB_SEG(W_) case W_: bad |= check_segment<Rule, W_>(kThreads, msg_bytes, BaseFromParams{args}, lo, hi, my_syn, rbit, cap); break;
-#define QLB_SEGW(W_) case W_: { const uint32_t rv = check_segment_wide<Rule, W_>(kThreads, msg_bytes, s_base4, lo, hi, my_syn, rbit, cap); bad |= rv & 1u; rbit = (int)(rv >> 1); } break;
+#define QLB_SEG(W_) case W_: bad |= check_segment<Rule, W_>(kThreads, msg_bytes, BaseFromParams{args}, lo, hi, my_syn, rbit, rule_arg); break;
+#define QLB_SEGW(W_) case W_: { const uint32_t rv = check_segment_wide<Rule, W_>(kThreads, msg_bytes, s_base4, lo, hi, my_syn, rbit, rule_arg); bad |= rv & 1u; rbit = (int)(rv >> 1); } break;
                             QLB_SEG(1) QLB_SEG(2) QLB_SEG(3) QLB_SEG(4) QLB_SEG(5) QLB_SEG(6) QLB_SEG(7) QLB_SEG(8)
                             QLB_SEGW(9) QLB_SEGW(10) QLB_SEGW(11) QLB_SEGW(12) QLB_SEGW(13) QLB_SEGW(14) QLB_SEGW(15) QLB_SEGW(16)
 #undef QLB_SEG

@@ -112,7 +112,7 @@ namespace qlb
     // row_stride: floats between the rows of consecutive slots (G, or B * G when B groups are interleaved slot by slot)
     template <typename Rule, int W, int VEC>
     __device__ __forceinline__ void stream_check(float *__restrict__ msg, const CodeDev &code, uint32_t p, int lane, uint32_t *__restrict__ synT,
-                                                 float cap, bool first, uint32_t (&bad)[VEC], uint32_t row_stride)
+                                                 typename Rule::Arg cap, bool first, uint32_t (&bad)[VEC], uint32_t row_stride)
     {
         float v[VEC][W];
         float *row[W];

@@ -361,7 +361,7 @@ namespace qlb
 #define QLB_PSEG(W_)                                                                                                          \
     case W_:                                                                                                                  \
         if constexpr (P::kLsbDecision)                                                                                        \
-            stream_check<typename P::Rule, W_, VEC>(msg, code, p, lane, sg.synT, cap, first, bad, rs);                        \
+            stream_check<typename P::Rule, W_, VEC>(msg, code, p, lane, sg.synT, P::Rule::check_arg(cap, args.ms_scale), first, bad, rs); \
         else                                                                                                                  \
             stream_check64<typename P::Math, W_, VEC>(msg, code, p, lane, sg.synT, bitsT, thr_eff, want_inf, first, bad, rs); \
         break;

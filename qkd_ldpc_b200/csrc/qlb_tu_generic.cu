@@ -50,9 +50,9 @@ namespace qlb
 
     int launch_generic(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        static const char *const kRuleName[] = {"f64", "f64fused", "f32", "f32fast"}; // indexed by Rule
+        static const char *const kRuleName[] = {"f64", "f64fused", "f32", "f32fast", "f32minsum"}; // indexed by Rule
         const char *name = kRuleName[(int)r.rule];
-        return with_rule<Rule::F64, Rule::F64Fused, Rule::F32, Rule::F32Fast>(r, [&](auto rule, auto reconcile) -> int
+        return with_rule<Rule::F64, Rule::F64Fused, Rule::F32, Rule::F32Fast, Rule::F32MinSum>(r, [&](auto rule, auto reconcile) -> int
         {
             typedef MathOf<decltype(rule)::value> Math;
             constexpr bool kReconcile = decltype(reconcile)::value;

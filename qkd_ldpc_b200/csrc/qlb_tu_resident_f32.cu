@@ -49,7 +49,8 @@ namespace
         QLB_CUDA(cudaMemcpyToSymbolAsync(g_bounds_msg_bytes, &msg_bytes, 4, 0, cudaMemcpyHostToDevice, ctx->stream));
 #endif
         char name[sizeof(qlb_ctx::last_decoder)];
-        std::snprintf(name, sizeof name, "resident_f32%s bw=%d threads=%d", std::is_same<CheckRule, RuleF32Fast>::value ? "fast" : "", kBW, kThreads);
+        const char *rule = std::is_same<CheckRule, RuleF32Fast>::value ? "fast" : std::is_same<CheckRule, RuleF32MinSum>::value ? "minsum" : "";
+        std::snprintf(name, sizeof name, "resident_f32%s bw=%d threads=%d", rule, kBW, kThreads);
         return launch_persistent(ctx, args, kern, kThreads, smem, 1, 0, name); // one resident CTA per SM
     }
 }
@@ -64,9 +65,9 @@ namespace qlb
 
     int launch_resident_f32(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        return with_rule<Rule::F32, Rule::F32Fast>(r, [&](auto rule, auto reconcile) -> int
+        return with_rule<Rule::F32, Rule::F32Fast, Rule::F32MinSum>(r, [&](auto rule, auto reconcile) -> int
         {
-            typedef std::conditional_t<decltype(rule)::value == Rule::F32Fast, RuleF32Fast, RuleF32Accurate> CheckRule;
+            typedef std::tuple_element_t<(int)decltype(rule)::value - (int)Rule::F32, std::tuple<RuleF32Accurate, RuleF32Fast, RuleF32MinSum>> CheckRule;
             constexpr bool kReconcile = decltype(reconcile)::value;
             switch (args.code.uniform_bit_w)
             {

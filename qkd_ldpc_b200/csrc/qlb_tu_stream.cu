@@ -125,7 +125,8 @@ namespace
 
     // The streaming kernels' form of each rule (qlb_stream_common.cuh).
     template <Rule kRule>
-    using StreamOf = std::tuple_element_t<(int)kRule, std::tuple<StreamF64<MathF64>, StreamF64<MathF64Fused>, StreamF32<RuleF32Accurate>, StreamF32<RuleF32Fast>>>;
+    using StreamOf = std::tuple_element_t<(int)kRule, std::tuple<StreamF64<MathF64>, StreamF64<MathF64Fused>, StreamF32<RuleF32Accurate>, StreamF32<RuleF32Fast>,
+                                                              StreamF32<RuleF32MinSum>>>;
 }
 namespace qlb
 {
@@ -137,7 +138,7 @@ namespace qlb
     }
     int launch_stream(qlb_ctx *ctx, DecodeArgs &args, const Route &r)
     {
-        return with_rule<Rule::F64, Rule::F64Fused, Rule::F32, Rule::F32Fast>(r, [&](auto rule, auto reconcile) -> int
+        return with_rule<Rule::F64, Rule::F64Fused, Rule::F32, Rule::F32Fast, Rule::F32MinSum>(r, [&](auto rule, auto reconcile) -> int
         {
             typedef StreamOf<decltype(rule)::value> P;
             constexpr bool kReconcile = decltype(reconcile)::value;

@@ -79,6 +79,17 @@ config_data get_config_data(fs::path config_path)
         }
         if (root.contains("device_fp32_fast_math"))
             cfg.DEVICE_FP32_FAST = root.at("device_fp32_fast_math").as_bool();
+        if (root.contains("device_fp32_min_sum_scale"))
+        {
+            cfg.DEVICE_FP32_MIN_SUM_SCALE = root.at("device_fp32_min_sum_scale").as_double();
+            if (cfg.DEVICE_FP32_MIN_SUM_SCALE != 0.) // 0: off
+            {
+                if (!(cfg.DEVICE_FP32_MIN_SUM_SCALE > 0. && cfg.DEVICE_FP32_MIN_SUM_SCALE <= 1.))
+                    throw std::runtime_error("device_fp32_min_sum_scale must be 0 (off) or in (0, 1]!");
+                if (cfg.DEVICE_PRECISION != 32 || cfg.DEVICE_FP32_FAST)
+                    throw std::runtime_error("device_fp32_min_sum_scale needs device_precision 32 and no device_fp32_fast_math!");
+            }
+        }
         if (root.contains("device_fp64_fused_ratio"))
             cfg.DEVICE_FP64_FUSED = root.at("device_fp64_fused_ratio").as_bool();
         if (root.contains("device_gpus"))

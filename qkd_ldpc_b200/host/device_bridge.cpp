@@ -132,6 +132,11 @@ namespace qkd_b200
         p.flags = (p.precision == QLB_PRECISION_F32 && CFG.DEVICE_FP32_FAST) ? QLB_FLAG_F32_FAST_MATH : 0;
         if (p.precision == QLB_PRECISION_F64 && CFG.DEVICE_FP64_FUSED)
             p.flags |= QLB_FLAG_F64_FUSED_RATIO;
+        if (CFG.DEVICE_FP32_MIN_SUM_SCALE != 0.) // config.cpp admits it with fp32 and without the fast rule only
+        {
+            p.flags |= QLB_FLAG_F32_MIN_SUM;
+            p.min_sum_scale = static_cast<float>(CFG.DEVICE_FP32_MIN_SUM_SCALE);
+        }
         return p;
     }
 }

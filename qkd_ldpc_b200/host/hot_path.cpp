@@ -56,6 +56,7 @@ namespace
         qlb_decode_params p = qkd_b200::params_from_cfg(max_it, thr);
         p.precision = QLB_PRECISION_F64; // the trace exists for the reference's arithmetic only
         p.flags = 0;
+        p.min_sum_scale = 0.f;
         const size_t n = h.num_bit_nodes, m = h.num_check_nodes;
         size_t edges = 0;
         for (size_t j = 0; j < m; ++j)

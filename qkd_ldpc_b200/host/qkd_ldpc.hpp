@@ -74,6 +74,7 @@ struct config_data
     // ---- additions of this implementation; every one defaults so that an unmodified reference config.json runs ----
     int DEVICE_PRECISION = 64;     // "device_precision": 64 (the reference's arithmetic) | 32
     bool DEVICE_FP32_FAST = false; // "device_fp32_fast_math": SFU check rule for fp32
+    double DEVICE_FP32_MIN_SUM_SCALE = 0.; // "device_fp32_min_sum_scale": 0 = off, else the normalized min-sum scale in (0, 1] (QLB_FLAG_F32_MIN_SUM)
     bool DEVICE_FP64_FUSED = false; // "device_fp64_fused_ratio": one-division form of the fp64 check rule (QLB_FLAG_F64_FUSED_RATIO)
     int DEVICE_GPUS = 0;           // "device_gpus": 0 = all visible GPUs
     size_t DEVICE_BATCH_FRAMES = 32768; // "device_batch_frames": most frames per launch handed to one GPU (the on-device key generator needs

@@ -55,7 +55,7 @@ namespace qkd_b200
         std::ofstream out(target, std::ios::out | std::ios::trunc);
         out << "SIM;MATRIX_FILENAME;M;N;QBER;FRAMES;SECONDS;FRAMES_PER_S;SIFTED_MBIT_PER_S;FRAME_ITERATIONS;MEAN_ITERATIONS;"
                "EFFICIENCY_F;LEAKED_BITS_PER_FRAME;GPUS;PRECISION\n";
-        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
+        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : CFG.DEVICE_FP32_MIN_SUM_SCALE != 0. ? "fp32-min-sum" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
         for (const point_report &p : report.points)
         {
             const double q = p.exact_qber, h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q);
@@ -302,7 +302,7 @@ namespace
     std::string report_row(const qkd_b200::point_report &p, int gpus)
     {
         std::ostringstream out;
-        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
+        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : CFG.DEVICE_FP32_MIN_SUM_SCALE != 0. ? "fp32-min-sum" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
         const double q = p.exact_qber, h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q);
         const double fps = p.seconds > 0 ? p.frames / p.seconds : 0.;
         out << p.sim_number << ";" << p.matrix_filename << ";" << p.num_check_nodes << ";" << p.num_bit_nodes << ";" << q << ";" << p.frames << ";"
