@@ -44,7 +44,8 @@ def test_multi_rate_codes_match_oracle(ctx, oracle, m, qs):
 
 
 def test_large_block_length_matches_oracle(ctx, oracle):
-    """N = 100 000 (E = 300 000): messages, indices and hard decisions live in per-CTA global scratch (tier 2)."""
+    """N = 100 000 (E = 300 000, 300 000 message slots): both precisions go to the streaming decoder, which takes every fp64 code
+    with 65 535 or more slots; three frames take its 32-frame-group form (vec=1, one bundle of one group, no repack)."""
     n, m = 100000, 51080
     mat = codes.peg_code(n, m, 3, 666, bfs_limit=2000)
     g, code = graph_of(mat), capi.Code.from_graph(mat)
@@ -55,6 +56,7 @@ def test_large_block_length_matches_oracle(ctx, oracle):
         for precision in (64, 32):
             it, res, dec, syn = ctx.reconcile_packed(code, capi.make_params(precision, mi, 100.0, True), capi.pack_bits(A), capi.pack_bits(B), Q,
                                                      want_syndrome=True)
+            assert ctx.last_decoder.startswith(f"stream_f{precision} vec=1 bw=3 bundle=1 waves=1"), ctx.last_decoder
             want_syn = np.stack([oracle.syndrome(g, a) for a in A])
             assert (capi.unpack_bits(syn, m) == want_syn).all()
             assert ((res & 1) == want[:, 1]).all() and (((res >> 1) & 1) == want[:, 2]).all()
@@ -97,6 +99,16 @@ def test_streaming_kernel_equals_resident_kernel(ctx, oracle, norepack):
     assert all((x == y).all() for x, y in zip(r, s))
 
 
+def assert_several_repacks(iterations, G, max_it):
+    """the streaming decoder repacked at least twice: restated from the iteration counts, under the kernel's round convention
+    and under r - 1 (test_gpu_stream_scale.repack_schedule)"""
+    from test_gpu_stream_scale import repack_schedule
+    groups = (len(iterations) + G - 1) // G
+    for lag in (0, 1):
+        sched = repack_schedule(iterations, G, groups, max_it, lag=lag)
+        assert len(sched) >= 2, sched
+
+
 def test_streaming_compaction_many_groups(ctx, oracle):
     """1 100 frames of the N=10240 code (9 groups = 3 bundles of 4, the last one partial and ragged) drawn by the on-device
     reference generator at QBERs that converge at very different rounds: the streaming decoder repacks the live frames
@@ -119,6 +131,8 @@ def test_streaming_compaction_many_groups(ctx, oracle):
     assert (r[0] == s[0]).all(), np.flatnonzero(r[0] != s[0])[:10]
     assert (r[1] == s[1]).all() and (r[2] == s[2]).all() and (r[3] == s[3]).all()
     assert 0 < int((r[1] & 1).sum()) < len(Q)  # the batch really mixes converging and failing frames
+    assert ctx.last_decoder.startswith("stream_f32 vec=4 bw=3 bundle=4 waves=1 repack=1"), ctx.last_decoder
+    assert_several_repacks(s[0], 128, 100)
     # sum-product entry (LLRs + target syndromes, no keys) through the same repacks; the priors are products here, which every
     # fp32 kernel rounds on their own (__fmul_rn) -- a contraction into the first sum would make the chaotic, non-converging
     # frames end on different last decisions in different kernels
@@ -219,6 +233,9 @@ def test_streaming_fp64_equals_resident_kernel(ctx, oracle, fused):
         s = ctx.reconcile_packed(code, capi.make_params(64, 100, 100.0, True, fast_math=fused, tier=3, **kw), A, B, Q, want_decoded=True, want_syndrome=True)
         assert (r[0] == s[0]).all(), (kw, np.flatnonzero(r[0] != s[0])[:10])
         assert all((x == y).all() for x, y in zip(r[1:], s[1:])), kw
+        if not kw:
+            assert ctx.last_decoder.startswith("stream_f64 vec=2 bw=3 bundle=4 waves=1 repack=1"), ctx.last_decoder
+            assert_several_repacks(s[0], 64, 100)
     # <= 32 frames: the 32-frame-group instantiation; and the clamp off (saturated products -> inf -> NaN totals, :508-524)
     for thr_on in (True, False):
         r21 = ctx.reconcile_packed(code, capi.make_params(64, 40, 100.0, thr_on, fast_math=fused), A[:21], B[:21], Q[:21], want_decoded=True, want_syndrome=True)
