@@ -35,8 +35,9 @@ extern "C" {
 #endif
 
 /* 0.2.0: qlb_decode_params grew execution knobs (was 24 bytes, now 40);
- * 0.3.0: QLB_FLAG_F32_MIN_SUM, and qlb_decode_params.reserved became min_sum_scale (same size and offsets) */
-#define QLB_VERSION 300
+ * 0.3.0: QLB_FLAG_F32_MIN_SUM, and qlb_decode_params.reserved became min_sum_scale (same size and offsets);
+ * 0.4.0: rate-adaptive reconciliation (qlb_rate_pattern, qlb_reconcile_adapted_packed, qlb_run_trials_adapted) */
+#define QLB_VERSION 400
 
 /* status codes (0 = ok); qlb_last_error() gives the message of the calling thread's last failure */
 enum {
@@ -239,6 +240,55 @@ int qlb_generate_device(qlb_ctx *ctx, int32_t n_bits, int64_t n_frames, const ui
  * only 8 bytes per frame go up and 5 come back. Host buffers. */
 int qlb_run_trials(qlb_ctx *ctx, const qlb_code *code, const qlb_decode_params *params, int64_t n_frames, const uint64_t *seeds,
                    uint64_t seed_offset, double qber, uint32_t *iterations_out, uint8_t *result_out, double *exact_qber_out);
+
+/* ---- rate-adaptive reconciliation (no reference counterpart) ----------------------------------------------------------
+ * One mother code of N bits and M checks, modulated per QBER (Elkouss, Martinez-Mateo, Lancho, Martin 2010): p PUNCTURED
+ * positions carry random bits of Alice's that Bob knows nothing about, s SHORTENED positions carry bits Alice reveals, the other
+ * n = N - p - s positions carry the key. A frame leaks M - p bits for an n-bit key: the effective rate is (N - M - s) / (N - p - s).
+ * pos_class[N] gives each position's class. Each call uploads and scans it (there is no pattern handle); it must hold only the
+ * three values below and at least one key position.
+ *
+ * A batch is turned, on the device, into the LLR-and-syndrome form of qlb_sum_product_batch and decoded there by the decoder
+ * and rule it would pick for that form (qlb_ctx_last_decoder names it); the key positions are then compared on the device:
+ *   - key bit k (0 <= k < n) sits at the k-th key position in ascending order; its prior is +-ln((1-q)/q) from Bob's bit (positive
+ *     for 0), ln((1-q)/q) formed in double on the host from qber[f] as qlb_reconcile_batch_packed forms it;
+ *   - fill bit k (0 <= k < p + s) sits at the k-th non-key position in ascending order, punctured and shortened alike; a punctured
+ *     position has prior +0.0, a shortened one +-threshold (positive for 0) -- finite, and no message can exceed it, so s > 0
+ *     requires enable_threshold (QLB_ERR_INVALID otherwise);
+ *   - Alice's mother word is her key and fill scattered the same way; the target syndrome is its syndrome;
+ *   - iterations_out and QLB_RES_SYNDROMES_MATCH are the decoder's; QLB_RES_KEYS_MATCH is set when the decoded bits equal Alice's
+ *     at every key position, independently of the syndrome flag (as the reference's arrays_equal);
+ *   - rules: s > 0 is accepted for every rule. p > 0 needs a check rule defined at a zero message: fp32 (leave-one-out products)
+ *     and fp32 min-sum. fp64 and fp64 fused divide by the edge's own tanh(m/2) and give 0/0 on a punctured edge (the reference's
+ *     QBER = 0.5 corner), fp32 fast math gives (S-D)/(D-S) = 0/0: they fail with QLB_ERR_UNSUPPORTED.
+ * Device staging is 8 N bytes of LLRs plus the packed words per frame: the caller's batch size bounds it.
+ */
+enum { QLB_POS_KEY = 0, QLB_POS_PUNCTURED = 1, QLB_POS_SHORTENED = 2 };
+
+/* Host only (no device, no context): the pattern of a mother code for p = n_punctured, s = n_shortened, into class_out[N].
+ * r_j is the j-th output (j = 0 ... N-1) of XoshiroCpp::Xoshiro256PlusPlus(seed) (seeded through SplitMix64, as the key generator).
+ * Positions are ordered by (r_j, j) ascending. Walking that order, position i is punctured when none of its checks already has a
+ * punctured bit (greedy untainted puncturing: every check holds at most one punctured bit, so each one is recovered in one step),
+ * until p are punctured; when the walk ends with fewer, QLB_ERR_UNSUPPORTED and the message gives the number available. Then the
+ * first s positions of the same order that are not punctured are shortened. With one seed the punctured sets for growing p are
+ * prefixes of one another (rate-compatible). Requires p, s >= 0 and p + s < N (QLB_ERR_INVALID). */
+int qlb_rate_pattern(const qlb_code *code, int32_t n_punctured, int32_t n_shortened, uint64_t seed, uint8_t *class_out);
+
+/* Host buffers. Keys are n-bit packed frames (ceil(n/32) words); fill_packed holds Alice's bits at the p + s non-key positions in
+ * ascending position order, ceil((p+s)/32) words per frame (may be NULL when p + s = 0); qber[f] is the exact error ratio over the
+ * n key bits, in (0, 1); qber[f] == 0 fails with QLB_ERR_KEY_TOO_SMALL ("Key size 'n' is too small for QBER.").
+ * decoded_key_packed_out (n-bit frames, the decoded bits at the key positions) may be NULL. */
+int qlb_reconcile_adapted_packed(qlb_ctx *ctx, const qlb_code *code, const qlb_decode_params *params, const uint8_t *pos_class,
+                                 int64_t n_frames, const uint32_t *alice_key_packed, const uint32_t *bob_key_packed,
+                                 const uint32_t *fill_packed, const double *qber, uint32_t *iterations_out, uint8_t *result_out,
+                                 uint32_t *decoded_key_packed_out);
+
+/* qlb_run_trials for a rate-adapted batch: 8 bytes up and 5 down per frame. Alice's and Bob's n-bit keys are exactly
+ * qlb_generate_batch_packed's at n_bits = n (floor(n * qber) errors; *exact_qber_out receives that count / n), and fill bit k is
+ * the top bit of the k-th output of Xoshiro256PlusPlus(~(seeds[f] + seed_offset)). */
+int qlb_run_trials_adapted(qlb_ctx *ctx, const qlb_code *code, const qlb_decode_params *params, const uint8_t *pos_class,
+                           int64_t n_frames, const uint64_t *seeds, uint64_t seed_offset, double qber, uint32_t *iterations_out,
+                           uint8_t *result_out, double *exact_qber_out);
 
 /* Test probe (no reference counterpart): the fp64 building blocks of the check rule, element-wise over host arrays, so that
  * their accuracy against the host libm is a test and not a claim. op 0: a / b (the rule's own division), 1: e^a for a in

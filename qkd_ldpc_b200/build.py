@@ -46,7 +46,8 @@ def _run(cmd, log: Path):
         raise RuntimeError(f"build failed: {' '.join(str(c) for c in cmd)}")
 
 
-TRANSLATION_UNITS = ["qlb_api.cu", "qlb_tu_generic.cu", "qlb_tu_resident_f32.cu", "qlb_tu_stream.cu", "qlb_tu_resident_f64.cu"]
+TRANSLATION_UNITS = ["qlb_api.cu", "qlb_tu_generic.cu", "qlb_tu_resident_f32.cu", "qlb_tu_stream.cu", "qlb_tu_resident_f64.cu",
+                     "qlb_rate.cu"]
 
 
 def build_library(force: bool = False, verbose_ptxas: bool = True, out: Path = LIB_PATH, extra_flags=()) -> Path:

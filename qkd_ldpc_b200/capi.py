@@ -20,6 +20,7 @@ FLAG_F64_FUSED_RATIO = 2
 FLAG_F32_MIN_SUM = 4
 RES_SYNDROMES_MATCH = 1
 RES_KEYS_MATCH = 2
+POS_KEY, POS_PUNCTURED, POS_SHORTENED = 0, 1, 2
 
 EXPORTS = [
     "qlb_version", "qlb_last_error", "qlb_device_count",
@@ -31,6 +32,7 @@ EXPORTS = [
     "qlb_syndrome_batch", "qlb_syndrome_batch_packed", "qlb_sum_product_batch", "qlb_sum_product_trace",
     "qlb_reconcile_batch", "qlb_reconcile_batch_packed", "qlb_reconcile_device", "qlb_stats_allreduce", "qlb_stats_comm_prepare",
     "qlb_generate_batch_packed", "qlb_generate_device", "qlb_run_trials", "qlb_test_f64_math",
+    "qlb_rate_pattern", "qlb_reconcile_adapted_packed", "qlb_run_trials_adapted",
 ]
 
 
@@ -107,6 +109,9 @@ def load_library(path: Path | None = None) -> C.CDLL:
     lib.qlb_generate_device.argtypes = [vp, i32, i64, vp, C.c_uint64, C.c_double, vp, vp, dp]
     lib.qlb_run_trials.argtypes = [vp, vp, pp, i64, vp, C.c_uint64, C.c_double, vp, vp, dp]
     lib.qlb_test_f64_math.argtypes = [vp, C.c_int, i64, vp, vp, vp]
+    lib.qlb_rate_pattern.argtypes = [vp, i32, i32, C.c_uint64, vp]
+    lib.qlb_reconcile_adapted_packed.argtypes = [vp, vp, pp, vp, i64, vp, vp, vp, vp, vp, vp, vp]
+    lib.qlb_run_trials_adapted.argtypes = [vp, vp, pp, vp, i64, vp, C.c_uint64, C.c_double, vp, vp, dp]
     if path is None:
         _lib = lib
     return lib
@@ -204,6 +209,13 @@ class Code:
             self.close()
         except Exception:
             pass
+
+
+def rate_pattern(code: Code, n_punctured: int, n_shortened: int, seed: int) -> np.ndarray:
+    """qlb_rate_pattern: the class (POS_KEY / POS_PUNCTURED / POS_SHORTENED) of each of the code's N positions. Host only."""
+    out = np.zeros(code.n, np.uint8)
+    _check(code.lib, code.lib.qlb_rate_pattern(code.handle, int(n_punctured), int(n_shortened), int(seed), _ptr(out)))
+    return out
 
 
 class Context:
@@ -345,6 +357,31 @@ class Context:
         exact = C.c_double()
         _check(self.lib, self.lib.qlb_run_trials(self.handle, code.handle, C.byref(params), seeds.size, _ptr(seeds), int(seed_offset),
                                                  float(qber), _ptr(it), _ptr(res), C.byref(exact)))
+        return it, res, exact.value
+
+    # ---- rate-adaptive reconciliation (a pattern from rate_pattern) ------------------------------------------------------
+    def reconcile_adapted(self, code: Code, params: DecodeParams, pos_class, alice_key_packed, bob_key_packed, fill_packed, qber,
+                          want_decoded=True):
+        """n-bit packed keys, fill [F][ceil((p+s)/32)] (None when p + s = 0) -> (iterations, result, decoded key or None)."""
+        cls = np.ascontiguousarray(pos_class, np.uint8)
+        ap = np.ascontiguousarray(np.atleast_2d(alice_key_packed), np.uint32)
+        bp = np.ascontiguousarray(np.atleast_2d(bob_key_packed), np.uint32)
+        fp = None if fill_packed is None else np.ascontiguousarray(np.atleast_2d(fill_packed), np.uint32)
+        f = ap.shape[0]
+        q = np.ascontiguousarray(np.broadcast_to(np.asarray(qber, np.float64), (f,)))
+        it, res = np.zeros(f, np.uint32), np.zeros(f, np.uint8)
+        dec = np.zeros_like(ap) if want_decoded else None
+        _check(self.lib, self.lib.qlb_reconcile_adapted_packed(self.handle, code.handle, C.byref(params), _ptr(cls), f, _ptr(ap), _ptr(bp),
+                                                               _ptr(fp), _ptr(q), _ptr(it), _ptr(res), _ptr(dec)))
+        return it, res, dec
+
+    def run_trials_adapted(self, code: Code, params: DecodeParams, pos_class, seeds, qber, seed_offset=0):
+        cls = np.ascontiguousarray(pos_class, np.uint8)
+        seeds = np.ascontiguousarray(seeds, np.uint64)
+        it, res = np.zeros(seeds.size, np.uint32), np.zeros(seeds.size, np.uint8)
+        exact = C.c_double()
+        _check(self.lib, self.lib.qlb_run_trials_adapted(self.handle, code.handle, C.byref(params), _ptr(cls), seeds.size, _ptr(seeds),
+                                                         int(seed_offset), float(qber), _ptr(it), _ptr(res), C.byref(exact)))
         return it, res, exact.value
 
     def f64_math(self, op: int, a, b=None):

@@ -79,6 +79,11 @@ namespace
         *dst_out = d;
         return QLB_OK;
     }
+}
+
+namespace qlb
+{
+    const CodeLayout &layout_of(const qlb_code *code) { return code->L; }
 
     int get_device_code(qlb_ctx *ctx, const qlb_code *code, const CodeDev **out)
     {
@@ -217,6 +222,10 @@ namespace
         return QLB_OK;
     }
 
+}
+
+namespace
+{
     void pack_frames(const int32_t *bits, int64_t frames, int n, int words, uint32_t *out)
     {
         for (int64_t f = 0; f < frames; ++f)
@@ -353,7 +362,8 @@ extern "C"
             for (void *p : kv.second.allocs)
                 cudaFree(p);
         for (DevBuf *b : {&ctx->scratch, &ctx->in_a, &ctx->in_b, &ctx->in_q, &ctx->in_llr, &ctx->in_syn, &ctx->out_it,
-                          &ctx->out_res, &ctx->out_dec, &ctx->out_syn, &ctx->gen_perm, &ctx->gen_seeds})
+                          &ctx->out_res, &ctx->out_dec, &ctx->out_syn, &ctx->gen_perm, &ctx->gen_seeds, &ctx->rate_tab,
+                          &ctx->rate_fill, &ctx->rate_word, &ctx->rate_key})
             b->release();
         if (ctx->d_counters)
             cudaFree(ctx->d_counters);

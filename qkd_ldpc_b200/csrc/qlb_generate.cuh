@@ -28,7 +28,7 @@ namespace qlb
     struct Xoshiro256pp
     {
         uint64_t s0, s1, s2, s3;
-        __device__ __forceinline__ explicit Xoshiro256pp(uint64_t seed)
+        __host__ __device__ __forceinline__ explicit Xoshiro256pp(uint64_t seed)
         {
             uint64_t x = seed;
             s0 = splitmix(x);
@@ -36,15 +36,15 @@ namespace qlb
             s2 = splitmix(x);
             s3 = splitmix(x);
         }
-        static __device__ __forceinline__ uint64_t splitmix(uint64_t &x)
+        static __host__ __device__ __forceinline__ uint64_t splitmix(uint64_t &x)
         {
             uint64_t z = (x += 0x9e3779b97f4a7c15ULL);
             z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ULL;
             z = (z ^ (z >> 27)) * 0x94d049bb133111ebULL;
             return z ^ (z >> 31);
         }
-        static __device__ __forceinline__ uint64_t rotl(uint64_t v, int k) { return (v << k) | (v >> (64 - k)); }
-        __device__ __forceinline__ uint64_t next()
+        static __host__ __device__ __forceinline__ uint64_t rotl(uint64_t v, int k) { return (v << k) | (v >> (64 - k)); }
+        __host__ __device__ __forceinline__ uint64_t next()
         {
             const uint64_t out = rotl(s0 + s3, 23) + s0;
             const uint64_t t = s1 << 17;

@@ -1,7 +1,8 @@
 // Internal declarations shared by the translation units of libqkdldpc_b200.so (not part of the C-ABI).
 // The library is split into TUs that compile in parallel: qlb_api.cu (C-ABI, code/context management, syndrome, key generator,
 // trace) and one per decoder family, with its admission predicate and its launcher: qlb_tu_generic.cu, qlb_tu_resident_f32.cu,
-// qlb_tu_resident_f64.cu, qlb_tu_stream.cu. route_decode, below, chooses the family of a batch.
+// qlb_tu_resident_f64.cu, qlb_tu_stream.cu. route_decode, below, chooses the family of a batch. qlb_rate.cu turns rate-adapted
+// batches into the sum-product mode every family takes.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -79,6 +80,7 @@ struct qlb_ctx
     uint64_t launches = 0;
     std::map<uint64_t, qlb::DeviceCode> codes;
     qlb::DevBuf scratch, in_a, in_b, in_q, in_llr, in_syn, out_it, out_res, out_dec, out_syn, gen_perm, gen_seeds;
+    qlb::DevBuf rate_tab, rate_fill, rate_word, rate_key; // rate-adapted batches (qlb_rate.cu): class tables, fill, mother words, keys
     std::vector<double> host_logp;
     std::vector<uint32_t> host_pack_a, host_pack_b, host_pack_out;
     char last_decoder[128] = {}; // written by each decode launcher just before it launches (qlb_ctx_last_decoder)
@@ -86,6 +88,14 @@ struct qlb_ctx
 
 namespace qlb
 {
+    struct CodeLayout;
+    // qlb_api.cu: the host layout of a code, its device copy on a context, the parameter check every decode entry runs, and the
+    // syndrome of packed device frames
+    const CodeLayout &layout_of(const qlb_code *code);
+    int get_device_code(qlb_ctx *ctx, const qlb_code *code, const CodeDev **out);
+    int check_params(const qlb_decode_params *p);
+    int launch_syndrome(qlb_ctx *ctx, const CodeDev &dev, long long n_frames, const uint32_t *d_bits, uint32_t *d_out);
+
     // Opt a kernel in to the device's whole per-block shared memory. ALWAYS the same value for a given kernel -- the attribute belongs
     // to the function, not to the launch, and contexts are driven from several host threads at once: setting it to what the current
     // launch needs lets another thread's smaller request land between this thread's set and its launch ("invalid argument").

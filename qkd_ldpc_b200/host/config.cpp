@@ -102,6 +102,20 @@ config_data get_config_data(fs::path config_path)
             if (cfg.DEVICE_BATCH_FRAMES < 1)
                 throw std::runtime_error("device_batch_frames must be >= 1!");
         }
+        if (root.contains("device_rate_adaptation"))
+        {
+            const mini_json::value &ra = root.at("device_rate_adaptation");
+            cfg.DEVICE_RATE_ADAPTATION = true;
+            cfg.DEVICE_RATE_MODULATED_FRACTION = ra.at("modulated_fraction").as_double();
+            cfg.DEVICE_RATE_TARGET_EFFICIENCY = ra.at("target_efficiency").as_double();
+            cfg.DEVICE_RATE_PATTERN_SEED = ra.at("pattern_seed").as_size();
+            if (!(cfg.DEVICE_RATE_MODULATED_FRACTION >= 0. && cfg.DEVICE_RATE_MODULATED_FRACTION < 1.))
+                throw std::runtime_error("device_rate_adaptation.modulated_fraction must be: 0 <= fraction < 1!");
+            if (!(cfg.DEVICE_RATE_TARGET_EFFICIENCY > 0.))
+                throw std::runtime_error("device_rate_adaptation.target_efficiency must be > 0!");
+            if (cfg.INTERACTIVE_MODE || cfg.TRACE_QKD_LDPC || cfg.TRACE_SUM_PRODUCT || cfg.TRACE_SUM_PRODUCT_LLR)
+                throw std::runtime_error("device_rate_adaptation runs in batch mode only, without interactive_mode and traces!");
+        }
         return cfg;
     }
     catch (const std::exception &)

@@ -37,6 +37,7 @@ std::vector<fs::path> get_file_paths_in_directory(const fs::path &directory_path
 //   --gen <seed> <n> <qber>              prints the exact QBER and Alice's / Bob's keys of one trial
 //   --seeds <seed> <count>               prints raw xoshiro256++ outputs
 //   --peg <n> <m> <dv> <seed> <out> [lim] writes a seeded PEG code as alist (configs[3], configs[4] of BASELINE.json)
+//   --rate-split <n> <m> <qber> <delta> <f>  prints the punctured and shortened counts of device_rate_adaptation at that point
 static int inspect(int argc, char **argv)
 {
     const std::string mode = argv[1];
@@ -117,7 +118,14 @@ static int inspect(int argc, char **argv)
                                      std::strtoull(argv[5], nullptr, 10), argc == 8 ? std::strtoull(argv[7], nullptr, 10) : 4096, argv[6]);
         return EXIT_SUCCESS;
     }
-    std::cerr << "usage: qkd_ldpc_b200_sim [dir] | --peg <n> <m> <col_weight> <seed> <out.alist> [bfs_limit] | --dump-matrix <alist|dense> <file> | --time-load <alist|dense> <file> | --gen <seed> <n> <qber> | --seeds <seed> <count>\n";
+    if (mode == "--rate-split" && argc == 7)
+    {
+        const auto [p, s] = qkd_b200::rate_split(std::strtoull(argv[2], nullptr, 10), std::strtoull(argv[3], nullptr, 10), std::strtod(argv[4], nullptr),
+                                                 std::strtod(argv[5], nullptr), std::strtod(argv[6], nullptr));
+        std::cout << p << " " << s << "\n";
+        return EXIT_SUCCESS;
+    }
+    std::cerr << "usage: qkd_ldpc_b200_sim [dir] | --peg <n> <m> <col_weight> <seed> <out.alist> [bfs_limit] | --dump-matrix <alist|dense> <file> | --time-load <alist|dense> <file> | --gen <seed> <n> <qber> | --seeds <seed> <count> | --rate-split <n> <m> <qber> <delta> <f>\n";
     return EXIT_FAILURE;
 }
 

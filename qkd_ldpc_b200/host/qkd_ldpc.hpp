@@ -15,8 +15,10 @@
 // There is no CPU decoder behind these functions: they throw std::runtime_error when no B200 is usable.
 #pragma once
 #include <cstddef>
+#include <cstdint>
 #include <filesystem>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "XoshiroCpp.hpp"
@@ -80,6 +82,12 @@ struct config_data
     size_t DEVICE_BATCH_FRAMES = 32768; // "device_batch_frames": most frames per launch handed to one GPU (the on-device key generator needs
                                         // >= 32 k trials in flight to reach its 2.2 M frames/s: 4 096 -> 0.67 M, 16 384 -> 1.83 M; scripts/gen_timing2.py)
     bool DEVICE_FORCE_ALLREDUCE = false; // "device_force_allreduce": run the statistics all-reduce through NCCL even on one GPU (tests)
+    // "device_rate_adaptation": {"modulated_fraction": delta, "target_efficiency": f, "pattern_seed": u64} -- each (matrix, QBER) point
+    // punctures and shortens delta * N positions of the matrix to aim at efficiency f (qkd_b200::rate_split, qlb_rate_pattern)
+    bool DEVICE_RATE_ADAPTATION = false;
+    double DEVICE_RATE_MODULATED_FRACTION = 0.;
+    double DEVICE_RATE_TARGET_EFFICIENCY = 0.;
+    uint64_t DEVICE_RATE_PATTERN_SEED = 0;
 };
 
 extern config_data CFG;
@@ -158,6 +166,7 @@ namespace qkd_b200
         size_t frames{};
         size_t frame_iterations{}; // executed BP iterations summed over the frames
         double seconds{};          // wall time of the point (generation + transfers + decode, all GPUs)
+        size_t punctured{}, shortened{}; // rate adaptation: p and s of the point's pattern (0 without it)
     };
     struct sweep_report // throughput side-report of the last QKD_LDPC_batch_simulation (never written into the reference CSV)
     {
@@ -177,8 +186,12 @@ namespace qkd_b200
     // files are removed when the sweep completes and the caller writes the final ones. Empty (default): no progress files.
     void set_progress_directory(const fs::path &directory);
     // Side file next to the reference-format CSV: per-point throughput, sifted-key rate, reconciliation efficiency
-    // f = (1 - R) / h2(q) and leaked bits per frame (= M: plain syndrome coding). SURVEY.md 8f-3.
+    // f = (1 - R) / h2(q) and leaked bits per frame (= M: plain syndrome coding). SURVEY.md 8f-3. With rate adaptation the
+    // leak is M - p bits for an n = N - p - s bit key, f = (M - p) / (n h2(q)), and PUNCTURED;SHORTENED;KEY_BITS;EFFECTIVE_RATE follow.
     void write_report(const sweep_report &report, fs::path directory);
+    // The (punctured, shortened) split of the sweep's rate adaptation for a code of n bits and m checks at QBER q: D = round(delta n)
+    // modulated positions, s = clamp(round(sigma n), 0, D) with sigma = R0 - (1 - f h2(q)) (1 - delta), R0 = 1 - m / n, and p = D - s.
+    std::pair<size_t, size_t> rate_split(size_t n, size_t m, double q, double delta, double target_efficiency);
     // Non-fatal findings about a loaded matrix (unsorted adjacency lists, duplicate edges); SURVEY.md 8f-2.
     std::vector<std::string> matrix_warnings(const H_matrix &matrix);
     // Seeded PEG construction of a column-weight-`dv` code, written as an alist file (host/peg.cpp).

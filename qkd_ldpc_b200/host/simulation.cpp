@@ -21,6 +21,7 @@
 #include <random>
 #include <stdexcept>
 #include <thread>
+#include <tuple>
 
 #include "device_bridge.hpp"
 #include "qkd_ldpc.hpp"
@@ -37,11 +38,45 @@ namespace
     };
 
     [[noreturn]] void key_too_small(size_t n) { throw std::runtime_error("Key size '" + std::to_string(n) + "' is too small for QBER."); }
+
+    // Header and row of the side file (qkd_b200::write_report); the last four columns exist with rate adaptation only.
+    std::string report_header()
+    {
+        return std::string("SIM;MATRIX_FILENAME;M;N;QBER;FRAMES;SECONDS;FRAMES_PER_S;SIFTED_MBIT_PER_S;FRAME_ITERATIONS;MEAN_ITERATIONS;"
+                           "EFFICIENCY_F;LEAKED_BITS_PER_FRAME;GPUS;PRECISION") +
+               (CFG.DEVICE_RATE_ADAPTATION ? ";PUNCTURED;SHORTENED;KEY_BITS;EFFECTIVE_RATE\n" : "\n");
+    }
+    std::string report_row(const qkd_b200::point_report &p, int gpus)
+    {
+        std::ostringstream out;
+        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : CFG.DEVICE_FP32_MIN_SUM_SCALE != 0. ? "fp32-min-sum" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
+        const double q = p.exact_qber, h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q);
+        const double fps = p.seconds > 0 ? p.frames / p.seconds : 0.;
+        // key bits and leaked bits per frame: N and M with plain syndrome coding
+        const size_t key_bits = p.num_bit_nodes - p.punctured - p.shortened, leak = p.num_check_nodes - p.punctured;
+        out << p.sim_number << ";" << p.matrix_filename << ";" << p.num_check_nodes << ";" << p.num_bit_nodes << ";" << q << ";" << p.frames << ";"
+            << p.seconds << ";" << fps << ";" << fps * key_bits / 1e6 << ";" << p.frame_iterations << ";"
+            << static_cast<double>(p.frame_iterations) / p.frames << ";" << (static_cast<double>(leak) / key_bits) / h2 << ";"
+            << leak << ";" << gpus << ";" << precision;
+        if (CFG.DEVICE_RATE_ADAPTATION)
+            out << ";" << p.punctured << ";" << p.shortened << ";" << key_bits << ";"
+                << static_cast<double>(p.num_bit_nodes - p.num_check_nodes - p.shortened) / key_bits;
+        out << "\n";
+        return out.str();
+    }
 }
 
 namespace qkd_b200
 {
     const sweep_report &last_sweep_report() { return g_report; }
+
+    std::pair<size_t, size_t> rate_split(size_t n, size_t m, double q, double delta, double target_efficiency)
+    {
+        const double h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q), r0 = 1. - static_cast<double>(m) / n;
+        const long long d = std::llround(delta * n);
+        const long long s = std::clamp(std::llround((r0 - (1. - target_efficiency * h2) * (1. - delta)) * n), 0LL, d);
+        return {static_cast<size_t>(d - s), static_cast<size_t>(s)};
+    }
 
     void write_report(const sweep_report &report, fs::path directory)
     {
@@ -53,18 +88,9 @@ namespace qkd_b200
         for (size_t dup = 1; fs::exists(target); ++dup)
             target = directory / (stem + "_" + std::to_string(dup) + ".csv");
         std::ofstream out(target, std::ios::out | std::ios::trunc);
-        out << "SIM;MATRIX_FILENAME;M;N;QBER;FRAMES;SECONDS;FRAMES_PER_S;SIFTED_MBIT_PER_S;FRAME_ITERATIONS;MEAN_ITERATIONS;"
-               "EFFICIENCY_F;LEAKED_BITS_PER_FRAME;GPUS;PRECISION\n";
-        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : CFG.DEVICE_FP32_MIN_SUM_SCALE != 0. ? "fp32-min-sum" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
+        out << report_header();
         for (const point_report &p : report.points)
-        {
-            const double q = p.exact_qber, h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q);
-            const double fps = p.seconds > 0 ? p.frames / p.seconds : 0.;
-            out << p.sim_number << ";" << p.matrix_filename << ";" << p.num_check_nodes << ";" << p.num_bit_nodes << ";" << q << ";" << p.frames << ";"
-                << p.seconds << ";" << fps << ";" << fps * p.num_bit_nodes / 1e6 << ";" << p.frame_iterations << ";"
-                << static_cast<double>(p.frame_iterations) / p.frames << ";" << (static_cast<double>(p.num_check_nodes) / p.num_bit_nodes) / h2 << ";"
-                << p.num_check_nodes << ";" << report.gpus << ";" << precision << "\n";
-        }
+            out << report_row(p, report.gpus);
     }
 
     std::vector<std::string> matrix_warnings(const H_matrix &h)
@@ -297,20 +323,6 @@ namespace
     }
     const char *kCsvHeader = "№;MATRIX_FILENAME;TYPE;CODE_RATE;M;N;QBER;ITERATIONS_SUCCESSFUL_SP_MEAN;ITERATIONS_SUCCESSFUL_SP_STD_DEV;"
                              "ITERATIONS_SUCCESSFUL_SP_MIN;ITERATIONS_SUCCESSFUL_SP_MAX;RATIO_TRIALS_SUCCESSFUL_SP;RATIO_TRIALS_SUCCESSFUL_LDPC;FER\n";
-    const char *kReportHeader = "SIM;MATRIX_FILENAME;M;N;QBER;FRAMES;SECONDS;FRAMES_PER_S;SIFTED_MBIT_PER_S;FRAME_ITERATIONS;MEAN_ITERATIONS;"
-                                "EFFICIENCY_F;LEAKED_BITS_PER_FRAME;GPUS;PRECISION\n";
-    std::string report_row(const qkd_b200::point_report &p, int gpus)
-    {
-        std::ostringstream out;
-        const std::string precision = CFG.DEVICE_PRECISION == 32 ? (CFG.DEVICE_FP32_FAST ? "fp32-fast" : CFG.DEVICE_FP32_MIN_SUM_SCALE != 0. ? "fp32-min-sum" : "fp32") : (CFG.DEVICE_FP64_FUSED ? "fp64-fused" : "fp64");
-        const double q = p.exact_qber, h2 = -q * std::log2(q) - (1. - q) * std::log2(1. - q);
-        const double fps = p.seconds > 0 ? p.frames / p.seconds : 0.;
-        out << p.sim_number << ";" << p.matrix_filename << ";" << p.num_check_nodes << ";" << p.num_bit_nodes << ";" << q << ";" << p.frames << ";"
-            << p.seconds << ";" << fps << ";" << fps * p.num_bit_nodes / 1e6 << ";" << p.frame_iterations << ";"
-            << static_cast<double>(p.frame_iterations) / p.frames << ";" << (static_cast<double>(p.num_check_nodes) / p.num_bit_nodes) / h2 << ";"
-            << p.num_check_nodes << ";" << gpus << ";" << precision << "\n";
-        return out.str();
-    }
 }
 
 namespace qkd_b200
@@ -345,6 +357,8 @@ std::vector<sim_result> QKD_LDPC_batch_simulation(const std::vector<sim_input> &
         const sim_input *in;
         double qber, exact_qber;
         qlb_code *code;
+        size_t punctured = 0, shortened = 0;
+        std::vector<uint8_t> pos_class; // rate adaptation: qlb_rate_pattern of the point (empty without it)
         std::atomic<size_t> batches_left{0};
         std::atomic<uint64_t> device_ns{0};
     };
@@ -357,13 +371,29 @@ std::vector<sim_result> QKD_LDPC_batch_simulation(const std::vector<sim_input> &
         for (const sim_input &in : sim_in)
             for (const double q : in.QBER)
             {
-                const size_t n = in.matrix.num_bit_nodes;
+                point &p = points[pt];
+                p.code = qkd_b200::code_for(in.matrix);
+                if (CFG.DEVICE_RATE_ADAPTATION)
+                {
+                    std::tie(p.punctured, p.shortened) = qkd_b200::rate_split(in.matrix.num_bit_nodes, in.matrix.num_check_nodes, q, CFG.DEVICE_RATE_MODULATED_FRACTION,
+                                                                              CFG.DEVICE_RATE_TARGET_EFFICIENCY);
+                    if (p.punctured > 0 && (CFG.DEVICE_PRECISION != 32 || CFG.DEVICE_FP32_FAST))
+                        throw std::runtime_error("device_rate_adaptation punctures " + std::to_string(p.punctured) + " bits at QBER " + std::to_string(q) +
+                                                 ": puncturing needs device_precision 32 without device_fp32_fast_math (fp32 or fp32 min-sum)!");
+                    if (p.shortened > 0 && !CFG.ENABLE_SUM_PRODUCT_MSG_LLR_THRESHOLD)
+                        throw std::runtime_error("device_rate_adaptation shortens " + std::to_string(p.shortened) + " bits at QBER " + std::to_string(q) +
+                                                 ": shortening needs enable_sum_product_msg_llr_threshold!");
+                    p.pos_class.resize(in.matrix.num_bit_nodes);
+                    if (qlb_rate_pattern(p.code, static_cast<int32_t>(p.punctured), static_cast<int32_t>(p.shortened), CFG.DEVICE_RATE_PATTERN_SEED,
+                                         p.pos_class.data()) != QLB_OK)
+                        throw std::runtime_error(std::string("device_rate_adaptation: ") + qlb_last_error());
+                }
+                const size_t n = in.matrix.num_bit_nodes - p.punctured - p.shortened; // the key bits of a frame
                 if (static_cast<size_t>(n * q) == 0)
                     key_too_small(n); // the reference throws from inside the point's first trial (src/simulation.cpp:170-175)
-                points[pt].in = &in;
-                points[pt].qber = q;
-                points[pt].exact_qber = static_cast<double>(static_cast<size_t>(n * q)) / n; // introduce_errors' return value (:436-459)
-                points[pt].code = qkd_b200::code_for(in.matrix);
+                p.in = &in;
+                p.qber = q;
+                p.exact_qber = static_cast<double>(static_cast<size_t>(n * q)) / n; // introduce_errors' return value (:436-459)
                 ++pt;
             }
     }
@@ -398,6 +428,8 @@ std::vector<sim_result> QKD_LDPC_batch_simulation(const std::vector<sim_input> &
         pr.frames = trials;
         pr.frame_iterations = frame_iterations;
         pr.seconds = seconds;
+        pr.punctured = points[pt].punctured;
+        pr.shortened = points[pt].shortened;
         return pr;
     };
 
@@ -414,7 +446,7 @@ std::vector<sim_result> QKD_LDPC_batch_simulation(const std::vector<sim_input> &
         progress_csv.open(progress_csv_path, std::ios::out | std::ios::trunc);
         progress_report.open(progress_report_path, std::ios::out | std::ios::trunc);
         progress_csv << kCsvHeader << std::flush;
-        progress_report << kReportHeader << std::flush;
+        progress_report << report_header() << std::flush;
     }
     auto flush_point = [&](size_t pt, const uint64_t *stats, double seconds)
     {
@@ -560,8 +592,12 @@ std::vector<sim_result> QKD_LDPC_batch_simulation(const std::vector<sim_input> &
                     result.resize(b.frames);
                     const auto t0 = clock::now();
                     double exact = 0;
-                    const int rc = qlb_run_trials(ctx, p.code, &params, static_cast<int64_t>(b.frames), reinterpret_cast<const uint64_t *>(&seeds[b.first_trial]),
-                                                  b.point, p.qber, iterations.data(), result.data(), &exact);
+                    const uint64_t *trial_seeds = reinterpret_cast<const uint64_t *>(&seeds[b.first_trial]);
+                    const int rc = p.pos_class.empty()
+                                       ? qlb_run_trials(ctx, p.code, &params, static_cast<int64_t>(b.frames), trial_seeds, b.point, p.qber, iterations.data(),
+                                                        result.data(), &exact)
+                                       : qlb_run_trials_adapted(ctx, p.code, &params, p.pos_class.data(), static_cast<int64_t>(b.frames), trial_seeds, b.point,
+                                                                p.qber, iterations.data(), result.data(), &exact);
                     const uint64_t ns = std::chrono::duration_cast<std::chrono::nanoseconds>(clock::now() - t0).count();
                     device_ns += ns;
                     p.device_ns += ns;
