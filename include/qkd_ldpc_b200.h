@@ -293,7 +293,9 @@ int qlb_run_trials_adapted(qlb_ctx *ctx, const qlb_code *code, const qlb_decode_
 /* Test probe (no reference counterpart): the fp64 building blocks of the check rule, element-wise over host arrays, so that
  * their accuracy against the host libm is a test and not a claim. op 0: a / b (the rule's own division), 1: e^a for a in
  * [-64, 0], 2: ln(a / b) for 0 < b <= a, 3: tanh(a / 2), 4: 2 atanh(a) (b != 0: IEEE infinities at |a| = 1), 5: e^-|a| (the table-driven
- * form the check rules use). b may be NULL for the unary ops. */
+ * form the check rules use), 6: the whole fp64 check rule as the resident decoder runs it, on records of 8 doubles (n a multiple of 8):
+ * a = the check's W messages (3 <= W <= 8), b = {W, syndrome bit, clamp threshold or +inf}, out = the W outgoing messages.
+ * b may be NULL for the unary ops. */
 int qlb_test_f64_math(qlb_ctx *ctx, int op, int64_t n, const double *a, const double *b, double *out);
 
 /* ---- sweep statistics ---------------------------------------------------------------------------

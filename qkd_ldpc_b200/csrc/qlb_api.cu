@@ -41,6 +41,45 @@ namespace qlb
         }
         out[i] = r;
     }
+    // op 6: the whole check rule as the resident fp64 kernel runs it (MathF64::check_fast with the exp table in shared memory and
+    // want_inf routed at compile time), one check per record of 8 doubles: a = the W messages, b = {W, syndrome bit, thr_eff}
+    template <int W>
+    __device__ __forceinline__ void f64_rule_probe(const double *a, double s, double thr_eff, const double2 *s_tab, double *out)
+    {
+        double v[W];
+#pragma unroll
+        for (int k = 0; k < W; ++k)
+            v[k] = a[k];
+        if (!(thr_eff <= 700.))
+            MathF64::check_fast<W, true>(v, s != 0., thr_eff, s_tab);
+        else
+            MathF64::check_fast<W, false>(v, s != 0., thr_eff, s_tab);
+#pragma unroll
+        for (int k = 0; k < W; ++k)
+            out[k] = v[k];
+    }
+    __global__ void f64_rule_probe_kernel(long long checks, const double *__restrict__ a, const double *__restrict__ b, double *__restrict__ out)
+    {
+        __shared__ double2 s_tab[32];
+        if (threadIdx.x < 32)
+            s_tab[threadIdx.x] = f64m::kExpTab[threadIdx.x];
+        __syncthreads();
+        const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+        if (c >= checks)
+            return;
+        const double *x = a + 8 * c, *p = b + 8 * c;
+        double *o = out + 8 * c;
+        switch ((int)p[0])
+        {
+        case 3: f64_rule_probe<3>(x, p[1], p[2], s_tab, o); break;
+        case 4: f64_rule_probe<4>(x, p[1], p[2], s_tab, o); break;
+        case 5: f64_rule_probe<5>(x, p[1], p[2], s_tab, o); break;
+        case 6: f64_rule_probe<6>(x, p[1], p[2], s_tab, o); break;
+        case 7: f64_rule_probe<7>(x, p[1], p[2], s_tab, o); break;
+        case 8: f64_rule_probe<8>(x, p[1], p[2], s_tab, o); break;
+        default: break;
+        }
+    }
 }
 
 namespace
@@ -724,7 +763,7 @@ extern "C"
     // ---- test probe of the fp64 building blocks -----------------------------------------------------------------------------
     int qlb_test_f64_math(qlb_ctx *ctx, int op, int64_t n, const double *a, const double *b, double *out)
     {
-        if (!ctx || n < 0 || op < 0 || op > 5 || (n > 0 && (!a || !out)))
+        if (!ctx || n < 0 || op < 0 || op > 6 || (n > 0 && (!a || !out)) || (op == 6 && (n % 8 != 0 || !b)))
             return fail(QLB_ERR_INVALID, "qlb_test_f64_math: bad arguments");
         if (n == 0)
             return QLB_OK;
@@ -736,7 +775,12 @@ extern "C"
         QLB_CUDA(cudaMemcpyAsync(d_a, a, bytes, cudaMemcpyHostToDevice, ctx->stream));
         if (b)
             QLB_CUDA(cudaMemcpyAsync(d_b, b, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        f64_math_probe_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(op, n, d_a, d_b, d_o);
+        if (op == 6)
+            QLB_CUDA(cudaMemsetAsync(d_o, 0, bytes, ctx->stream)); // the slots of a record beyond its W messages come back as 0
+        if (op == 6)
+            f64_rule_probe_kernel<<<(unsigned)((n / 8 + 255) / 256), 256, 0, ctx->stream>>>(n / 8, d_a, d_b, d_o);
+        else
+            f64_math_probe_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(op, n, d_a, d_b, d_o);
         QLB_CUDA(cudaGetLastError());
         QLB_CUDA(cudaMemcpyAsync(out, d_o, bytes, cudaMemcpyDeviceToHost, ctx->stream));
         QLB_CUDA(cudaStreamSynchronize(ctx->stream));

@@ -36,7 +36,8 @@ namespace qlb
         static __constant__ double kLn2Hi = 6.93147180369123816490e-01, kLn2Lo = 1.90821492927058770002e-10;
         // 2^(j/32), j = 0 ... 31, as (leading double, remainder) pairs: the table of the table-driven exp below (P. T. P. Tang's scheme,
         // "Table-driven implementation of the exponential function in IEEE floating-point arithmetic", ACM TOMS 15, 1989; the values
-        // themselves computed here to 70 digits). Read with one 128-bit L1-cached load per call (512 B: always resident).
+        // themselves computed here to 70 digits). Read with one 128-bit L1-cached load per call (512 B: always resident), or from
+        // a copy in shared memory (the resident fp64 kernel).
         static __device__ const double2 kExpTab[32] = {
             {0x1.0000000000000p+0, 0x0.0p+0}, {0x1.059b0d3158574p+0, 0x1.d73e2a475b465p-55}, {0x1.0b5586cf9890fp+0, 0x1.8a62e4adc610bp-54},
             {0x1.11301d0125b51p+0, -0x1.6c51039449b3ap-54}, {0x1.172b83c7d517bp+0, -0x1.19041b9d78a76p-55}, {0x1.1d4873168b9aap+0, 0x1.e016e00a2643cp-54},
@@ -72,7 +73,8 @@ namespace qlb
         // (an infinity becomes 1024, a NaN some value in [1024, 1025): callers that can see a NaN track it themselves), and the
         // binary exponent k is kept above -1000 so that the integer exponent insertion cannot wrap: beyond |m| ~ 693 the result is
         // a positive number far below 2^-54 instead of e^-|m|, which is all tanh(|m| / 2) = (1 - e) / (1 + e) = 1 needs.
-        __device__ __forceinline__ double exp_neg_abs(double m)
+        // s_tab: a copy of kExpTab in shared memory (a 32-bit-addressed LDS.128 instead of a 64-bit address and an LDG), or null.
+        __device__ __forceinline__ double exp_neg_abs(double m, const double2 *s_tab = nullptr)
         {
             const double kMagic = 6755399441055744.0;
             const double a = __hiloint2double(min(__double2hiint(m) & 0x7fffffff, 0x40900000), __double2loint(m));
@@ -101,7 +103,7 @@ namespace qlb
             c = fma(r, c, kExpQ[3]);
             c = fma(r, c, 0.5);
             const double q = fma(r * r, c, r);
-            const double2 T = __ldg(&kExpTab[n & 31]);
+            const double2 T = s_tab ? s_tab[n & 31] : __ldg(&kExpTab[n & 31]);
             const double p = T.x + fma(T.x, q, T.y);
             return __hiloint2double(__double2hiint(p) + ((n >> 5) << 20), __double2loint(p));
 #endif
@@ -144,7 +146,7 @@ namespace qlb
 
         // ln(num / den) for 0 < den <= num without forming the quotient: ONE division for the ratio and the logarithm together.
         // den is rescaled by the power of two 2^j that brings m = num / (den 2^j) into ~[sqrt(1/2), sqrt 2] (exponent difference,
-        // corrected by one through an integer comparison of the leading mantissa bits; the boundary need not be exact, the
+        // corrected by one through a comparison of the leading mantissa bits; the boundary need not be exact, the
         // polynomial holds a little beyond it). Then s = (m - 1) / (m + 1) = (num - den') / (num + den') -- the numerator is exact
         // (Sterbenz) -- and ln m = 2 s + s R(s^2) with fdlibm's R (e_log.c: "log(1+f) = 2s + s*R"), result j ln 2 + ln m. <= 2 ulp.
         // (the special outcomes are selected by the caller from `num`, `den`: for operands outside 0 < den <= num the value
@@ -152,11 +154,15 @@ namespace qlb
         __device__ __forceinline__ double log_ratio(double num, double den)
         {
             const int hn = __double2hiint(num), hd = __double2hiint(den);
-            int j = (hn >> 20) - (hd >> 20);
-            // leading 16 mantissa bits (with the hidden one) of both: u / d in (1/2, 2)
-            const uint32_t u = (((uint32_t)hn & 0x000fffffu) | 0x00100000u) >> 5, d = (((uint32_t)hd & 0x000fffffu) | 0x00100000u) >> 5;
-            j += (u * 46341u > d * 65536u) ? 1 : 0; // u / d > sqrt 2
-            j -= (u * 65536u < d * 46341u) ? 1 : 0; // u / d < sqrt(1/2)
+            // The leading 16 mantissa bits (with the hidden one) of both, u and d, as the floats U = u 2^-15 and D = d 2^-15 in [1, 2).
+            // j = exponent difference + [u / d > sqrt 2] - [u / d < sqrt(1/2)], the two tests being u 46341 > d 65536 and
+            // u 65536 < d 46341. Each is the sign of ONE fp32 FMA: U c - D (c = 46341 / 65536, exact) is the rounding of the exact
+            // difference, rounding keeps the sign, and the difference is never zero (65536 would have to divide u 46341) -- so the
+            // sign bits give both tests without predicates, for every pair of high words (checked on all 2^30 pairs (u, d)).
+            const float U = __int_as_float(((hn << 3) & 0x007fff00) | 0x3f800000), D = __int_as_float(((hd << 3) & 0x007fff00) | 0x3f800000);
+            const uint32_t not_above = (uint32_t)__float_as_int(fmaf(U, 46341.f / 65536.f, -D)) >> 31; // 1: u / d < sqrt 2
+            const uint32_t not_below = (uint32_t)__float_as_int(fmaf(D, 46341.f / 65536.f, -U)) >> 31; // 1: u / d > sqrt(1/2)
+            const int j = (hn >> 20) - (hd >> 20) + (int)not_below - (int)not_above;
             const double ds = __hiloint2double(hd + (j << 20), __double2loint(den));
             const double s = div_pos(num - ds, num + ds);
             const double z = s * s;
@@ -181,9 +187,9 @@ namespace qlb
         // tanh(m / 2) = (1 - e^-|m|) / (1 + e^-|m|); |m| capped (exp_neg_abs; the quotient is exactly +-1 far earlier).
         // m = NaN comes back as +-1, NOT NaN: callers that can see a NaN message track it themselves (MathF64::check poisons the
         // row product, TwoPass<MathF64>::t passes the NaN through) so that the hot loop pays one compare instead of a select pair.
-        __device__ __forceinline__ double tanh_half(double m)
+        __device__ __forceinline__ double tanh_half(double m, const double2 *s_tab = nullptr)
         {
-            const double e = exp_neg_abs(m);
+            const double e = exp_neg_abs(m, s_tab);
             return copysign(div_any(1. - e, 1. + e), m);
         }
         // 2 atanh(p) = ln((1 + |p|) / (1 - |p|)) with p's sign, |p| <= 1 (the caller's p is a product of tanh values divided by one

@@ -185,10 +185,24 @@ namespace qlb
         }
         // The same rule for a check of weight exactly W with the clamp folded into its operands: thr_eff = the clamp, or +inf
         // when it is disabled (no magnitude exceeds it; a NaN fails the comparison and passes, :508-524); want_inf = the clamp is
-        // disabled or above ln(2^1024), i.e. a saturated product must come out as the IEEE infinity before the clamp.
+        // disabled or above ln(2^1024), i.e. a saturated product must come out as the IEEE infinity before the clamp. Without it
+        // a saturated product gives 1024 ln 2 > 700 >= thr_eff, which the clamp turns into thr_eff as it would the infinity.
         template <int W>
         static __device__ __forceinline__ void check_fast(double (&v)[W], bool s, double thr_eff, bool want_inf)
         {
+            check_rule<W, -1>(v, s, thr_eff, want_inf, nullptr);
+        }
+        // want_inf fixed at compile time (the resident kernel routes on it), s_exp_tab: f64m::kExpTab staged in shared memory
+        template <int W, bool kWantInf>
+        static __device__ __forceinline__ void check_fast(double (&v)[W], bool s, double thr_eff, const double2 *s_exp_tab)
+        {
+            check_rule<W, kWantInf ? 1 : 0>(v, s, thr_eff, kWantInf, s_exp_tab);
+        }
+        // kWantInf: 0 / 1 = want_inf known at compile time, -1 = the run-time value of `want_inf`
+        template <int W, int kWantInf>
+        static __device__ __forceinline__ void check_rule(double (&v)[W], bool s, double thr_eff, bool want_inf, const double2 *s_exp_tab)
+        {
+            want_inf = kWantInf < 0 ? want_inf : kWantInf == 1;
 #if !defined(QLB_F64_LIBM_FORMS)
             double row = s ? -1. : 1.;
             bool poisoned = false;
@@ -196,7 +210,7 @@ namespace qlb
             for (int k = 0; k < W; ++k)
             {
                 poisoned |= v[k] != v[k];
-                v[k] = tanh_half(v[k]);
+                v[k] = f64m::tanh_half(v[k], s_exp_tab);
                 row *= v[k];
             }
             row = poisoned ? __longlong_as_double(0x7ff8000000000000LL) : row;
@@ -212,6 +226,7 @@ namespace qlb
                 v[k] = copysign(r, q);
             }
 #else
+            (void)s_exp_tab;
             check<W>(v, W, s, thr_eff < __longlong_as_double(0x7ff0000000000000LL), thr_eff);
 #endif
         }
@@ -273,6 +288,17 @@ namespace qlb
         template <int W>
         static __device__ __forceinline__ void check_fast(double (&v)[W], bool s, double thr_eff, bool)
         {
+            check_rule<W>(v, s, thr_eff, nullptr);
+        }
+        // the resident kernel's form (see MathF64): want_inf does not apply, s_exp_tab = f64m::kExpTab in shared memory
+        template <int W, bool>
+        static __device__ __forceinline__ void check_fast(double (&v)[W], bool s, double thr_eff, const double2 *s_exp_tab)
+        {
+            check_rule<W>(v, s, thr_eff, s_exp_tab);
+        }
+        template <int W>
+        static __device__ __forceinline__ void check_rule(double (&v)[W], bool s, double thr_eff, const double2 *s_exp_tab)
+        {
             double e[W];
             double A = 1., B = 1.;
             uint32_t neg = s ? 0x80000000u : 0u;
@@ -282,7 +308,7 @@ namespace qlb
             {
                 poisoned |= v[k] != v[k];
                 neg ^= (uint32_t)__double2hiint(v[k]);
-                e[k] = f64m::exp_neg_abs(v[k]);
+                e[k] = f64m::exp_neg_abs(v[k], s_exp_tab);
                 A *= 1. - e[k];
                 B *= 1. + e[k];
             }

@@ -36,7 +36,7 @@ namespace qlb
 #endif
     constexpr int kResident64Threads = QLB_R64_THREADS; // launch bound (768: 80 registers)
     constexpr int kResident64FastW = 8;     // weights up to this get the split-specialised loops
-    constexpr size_t kResident64StaticSmem = 256;
+    constexpr size_t kResident64StaticSmem = 768; // s_base, s_frame, the exp table s_exp_tab (512 B), and the system's reserve
 
     // A group of the check walk: sorted positions p0 + l0 .. p0 + l1 (p0 a multiple of 32), all of weight w, the split falling
     // the same way for each: `tail` rows (edge positions w - tail .. w - 1) in the global tail (0 or 1), or 3: decide per access.
@@ -95,8 +95,9 @@ namespace qlb
     };
 
     // The check rule (:220-249) on the checks p0 + lane of one group.
-    template <typename Math, int W, int kTail, typename Base>
-    __device__ __forceinline__ void check_group64(const Split64 &msg, const Base s_base, uint32_t p, bool active, bool syn, double thr_eff, bool want_inf)
+    template <typename Math, bool kWantInf, int W, int kTail, typename Base>
+    __device__ __forceinline__ void check_group64(const Split64 &msg, const Base s_base, uint32_t p, bool active, bool syn, double thr_eff,
+                                                  const double2 *s_exp_tab)
     {
         if (!active)
             return;
@@ -113,7 +114,7 @@ namespace qlb
                 QLB_CHECK_INDEX(msg.smem_slots, slot + 1u); // ... and one it promises to the global tail
             v[k] = kTail == 3 ? msg.ld(slot) : (k < W - kTail ? msg.smem[slot] : gm[slot]);
         }
-        Math::template check_fast<W>(v, syn, thr_eff, want_inf);
+        Math::template check_fast<W, kWantInf>(v, syn, thr_eff, s_exp_tab);
 #pragma unroll
         for (int k = 0; k < W; ++k)
         {
@@ -128,10 +129,11 @@ namespace qlb
     }
     // Weights 9..16 (the R >= 0.7 codes of the CW = 3 family) are kept out of line: their register appetite (2 x W doubles live) must
     // not leak into the hot instantiations; some spilling inside them is still far cheaper than the generic kernel's L2 round trips.
-    template <typename Math, int W>
-    __device__ __noinline__ void check_group64_wide(const Split64 msg, const uint32_t *s_base, uint32_t p, bool active, bool syn, double thr_eff, bool want_inf)
+    template <typename Math, bool kWantInf, int W>
+    __device__ __noinline__ void check_group64_wide(const Split64 msg, const uint32_t *s_base, uint32_t p, bool active, bool syn, double thr_eff,
+                                                    const double2 *s_exp_tab)
     {
-        check_group64<Math, W, 3>(msg, Base64FromSmem{s_base}, p, active, syn, thr_eff, want_inf);
+        check_group64<Math, kWantInf, W, 3>(msg, Base64FromSmem{s_base}, p, active, syn, thr_eff, s_exp_tab);
     }
 
     // Sorted position of the check that owns `slot` (rows are laid out one edge position after the other, qlb_layout.hpp).
@@ -149,13 +151,15 @@ namespace qlb
     }
 
     // kBW: uniform bit weight. Host-checked: slots < 65535, n < 65536, m < 65536, max_check_w <= 16, n % 32 == 0.
-    template <typename Math, bool kReconcile, int kBW, int kMaxThreads>
+    // kWantInf: the clamp is off or above 700, so a saturated check product must give the IEEE infinity (MathF64::check_fast).
+    template <typename Math, bool kReconcile, int kBW, int kMaxThreads, bool kWantInf>
     __global__ void __launch_bounds__(kMaxThreads, 1) decode_resident_f64_kernel(const DecodeArgs args)
     {
         const int kThreads = blockDim.x; // multiple of 32, <= kMaxThreads
         extern __shared__ __align__(16) unsigned char smem[];
         __shared__ uint32_t s_base[kResidentMaxCW];
         __shared__ long long s_frame;
+        __shared__ double2 s_exp_tab[32];
 
         const CodeDev &code = args.code;
         const int n = code.n, m = code.m, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, warps = kThreads >> 5;
@@ -180,6 +184,8 @@ namespace qlb
 
         if (tid < kResidentMaxCW)
             s_base[tid] = code.base[tid];
+        if (tid < 32)
+            s_exp_tab[tid] = f64m::kExpTab[tid];
         for (int g = tid; g < n_cg; g += kThreads)
             s_cg[g] = code.r64_check_group_table[g];
         for (int g = tid; g < n_bg; g += kThreads)
@@ -187,7 +193,6 @@ namespace qlb
         const uint16_t *bslot = code.bit_slots16;
         const double kInf = __longlong_as_double(0x7ff0000000000000LL);
         const double thr_eff = args.enable_thr ? args.thr : kInf; // the clamp as an operand: nothing exceeds +inf
-        const bool want_inf = !(thr_eff <= 700.);                  // a saturated product must be the IEEE infinity before the clamp
 
         for (;;)
         {
@@ -300,11 +305,11 @@ namespace qlb
                         switch (ent >> 21)
                         {
 #define QLB_GRP64(W_)                                                                                                       \
-    case W_ * 4 + 0: check_group64<Math, W_, 0>(msg, Base64FromParams{args}, p, active, syn, thr_eff, want_inf); break;     \
-    case W_ * 4 + 1: check_group64<Math, W_, 1>(msg, Base64FromParams{args}, p, active, syn, thr_eff, want_inf); break;     \
-    case W_ * 4 + 3: check_group64<Math, W_, 3>(msg, Base64FromParams{args}, p, active, syn, thr_eff, want_inf); break;
+    case W_ * 4 + 0: check_group64<Math, kWantInf, W_, 0>(msg, Base64FromParams{args}, p, active, syn, thr_eff, s_exp_tab); break; \
+    case W_ * 4 + 1: check_group64<Math, kWantInf, W_, 1>(msg, Base64FromParams{args}, p, active, syn, thr_eff, s_exp_tab); break; \
+    case W_ * 4 + 3: check_group64<Math, kWantInf, W_, 3>(msg, Base64FromParams{args}, p, active, syn, thr_eff, s_exp_tab); break;
 #define QLB_GRP64W(W_) \
-    case W_ * 4 + 3: check_group64_wide<Math, W_>(msg, s_base, p, active, syn, thr_eff, want_inf); break;
+    case W_ * 4 + 3: check_group64_wide<Math, kWantInf, W_>(msg, s_base, p, active, syn, thr_eff, s_exp_tab); break;
                             QLB_GRP64(1) QLB_GRP64(2) QLB_GRP64(3) QLB_GRP64(4) QLB_GRP64(5) QLB_GRP64(6) QLB_GRP64(7) QLB_GRP64(8)
                             QLB_GRP64W(9) QLB_GRP64W(10) QLB_GRP64W(11) QLB_GRP64W(12) QLB_GRP64W(13) QLB_GRP64W(14) QLB_GRP64W(15) QLB_GRP64W(16)
 #undef QLB_GRP64

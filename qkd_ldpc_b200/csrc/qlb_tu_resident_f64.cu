@@ -21,7 +21,13 @@ namespace
     template <typename Math, bool kReconcile, int kBW>
     int launch_resident64(qlb_ctx *ctx, DecodeArgs &args, int block_threads)
     {
-        auto kern = decode_resident_f64_kernel<Math, kReconcile, kBW, kResident64Threads>;
+        // the infinity of a saturated product is only materialised where the clamp cannot hide it (MathF64::check_fast); the fused
+        // rule produces it either way and has the one instantiation
+        const double thr_eff = args.enable_thr ? args.thr : __builtin_huge_val();
+        auto kern = decode_resident_f64_kernel<Math, kReconcile, kBW, kResident64Threads, false>;
+        if constexpr (std::is_same<Math, MathF64>::value)
+            if (!(thr_eff <= 700.))
+                kern = decode_resident_f64_kernel<Math, kReconcile, kBW, kResident64Threads, true>;
         const CodeDev &c = args.code;
         int kThreads = kResident64Threads;
         if (const int t = block_threads / 32 * 32) // qlb_decode_params.block_threads
